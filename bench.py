@@ -21,6 +21,9 @@ Prints ONE JSON line (rank 0).  `value` = candidates optimised per second, input
 (CUDA events), max over ranks.  `e2e` = the same through the host-buffer C ABI (alore_esdf_update + alore_opt_batch)
 with every copy inside the timed region.  The reference arm runs the CPU restatement on a bounded random sample of
 the SAME block with the ESDF cost amortised over the sample fraction, so both arms measure the same workload.
+
+`--dump-outputs DIR` (rank 0) writes what the last timed tick returned as DIR/<name>.npy (float64), see dump_outputs.
+The inputs depend on the arguments only, so two builds run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -37,6 +40,7 @@ from pathlib import Path
 
 import numpy as np
 
+sys.dont_write_bytecode = True     # the benchmark may run from a read-only tree and writes nothing into it
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
 
@@ -44,6 +48,8 @@ PER_GPU = 8320
 METRIC = "candidate trajs optimized/sec (ESDF Mcells/s under 'esdf')"
 UNIT = "trajs/s"
 SAMPLE = 2080                      # candidates of the rank-0 block the CPU arm optimises per step
+DUMP_LIMIT = 64 << 20              # bytes --dump-outputs writes at most, .npy headers included
+DUMP_ESDF_CELLS = 1 << 19          # ESDF cells --dump-outputs writes (a seeded sample of the 2048^2 map)
 
 
 def workload_config(per_gpu):
@@ -177,6 +183,35 @@ def sample_indices(n, k, seed=11):
     return np.sort(np.random.default_rng(seed).choice(n, size=min(k, n), replace=False))
 
 
+def dump_outputs(out_dir, res, cands, best, dist, limit=DUMP_LIMIT):
+    """--dump-outputs: the results of one tick as float64 .npy files under `out_dir`, `limit` bytes at most.
+
+    best_cost / best_index: the winner the step returns.  esdf_distance: the tick's ESDF at the cells listed in
+    esdf_cells (a seeded sample).  For the candidates listed in `candidates` (the whole block while it fits the limit,
+    else a seeded sample), in that order: ok, status, replans, alm_iters, evals, cost, tail_s (one value each) and their
+    pieces, piece_T [P], coeffs [P, 6, 2], inner_pts [P - len(candidates), 2]."""
+    rng = np.random.default_rng(0)
+    cells = np.sort(rng.choice(dist.size, size=min(DUMP_ESDF_CELLS, dist.size), replace=False))
+    room = limit - (1 << 20) - 8 * (2 + 2 * cells.size)          # 1 MB spare for the .npy headers
+    n = np.diff(cands.piece_off).astype(np.int64)
+    per_cand = 8 * (15 * n + 6)      # index + 7 scalars; 12 coefficients and one duration per piece; N - 1 inner points
+    keep = np.arange(cands.B)
+    if per_cand.sum() > room:
+        order = rng.permutation(cands.B)
+        keep = np.sort(order[:np.searchsorted(np.cumsum(per_cand[order]), room, side="right")])
+    po = cands.piece_off
+    pieces = np.concatenate([np.arange(0)] + [np.arange(po[b], po[b + 1]) for b in keep]).astype(np.int64)
+    inner = np.concatenate([np.arange(0)] + [np.arange(po[b] - b, po[b + 1] - b - 1) for b in keep]).astype(np.int64)
+    arrays = {"best_cost": [best[0]], "best_index": [best[1]], "esdf_cells": cells, "esdf_distance": dist[cells],
+              "candidates": keep, "piece_T": res.piece_T[pieces], "coeffs": res.coeffs[pieces], "inner_pts": res.inner_pts[inner]}
+    for f in ("ok", "status", "replans", "alm_iters", "evals", "cost", "tail_s"):
+        arrays[f] = getattr(res, f)[keep]
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", np.asarray(a, dtype=np.float64))
+
+
 def cpu_arm(steps, warmup, per_gpu):
     """The reference's CPU algorithm (oracle port; the real one needs ROS+Eigen+PCL and cannot be built here, see
     DESIGN.md) on all host threads: per step, one single-thread 2048^2 ESDF rebuild (the reference's ESDF is serial)
@@ -253,7 +288,10 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--per-gpu", type=int, default=PER_GPU)
     ap.add_argument("--skip-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed tick as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -418,7 +456,7 @@ def main():
     kern_ms = []
     e0.record(stream)
     for t in range(1 + args.warmup, n_ticks):
-        step_resident(t)
+        best = step_resident(t)
         kern_ms.append(batches[t].kernel_ms())
     e1.record(stream)
     barrier()
@@ -450,6 +488,9 @@ def main():
         step_e2e(t)
     barrier()
     e2e_s = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0:
+        # the resident loop's last tick; the e2e loop ended on the same tick and left its ESDF in the map's host buffer
+        dump_outputs(args.dump_outputs, res_last, ticks[-1][1], best, m.distance_buffer_all_)
 
     # ---- the heaviest candidate alone (what bounds a rank's step), ALM statistics ----------------------------------
     heavy = int(np.argmax(res_last.evals * np.diff(ticks[-1][1].piece_off)))
