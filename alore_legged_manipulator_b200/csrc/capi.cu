@@ -237,7 +237,9 @@ int alore_esdf_update_dev(alore_ctx* ctx, const alore_map_geom_t* geom, const ui
     // device, what alore_esdf_update does from the host) and the resident ESDF is rebuilt
     if (!ctx->d_occ || !ctx->d_dist || (size_t)geom->glx * geom->gly != ctx->map_cells || std::memcmp(&ctx->geom, geom, sizeof(*geom)) != 0)
       return alore_fail(ctx, ALORE_ENOMAP, "no resident map of this geometry: call alore_esdf_update / alore_esdf_reset first");
-    if (min_x < 0 || max_x >= geom->glx || max_x < min_x) return alore_fail(ctx, ALORE_EINVAL, "esdf window outside the grid");
+    // the whole window is checked before the copy: a refused call leaves the resident grid as it was
+    if (min_x < 0 || max_x >= geom->glx || max_x < min_x || min_y < 0 || max_y >= geom->gly || max_y < min_y)
+      return alore_fail(ctx, ALORE_EINVAL, "esdf window outside the grid");
     cudaStream_t st2 = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
     const size_t gly = geom->gly;
     ALORE_CUDA(ctx, cudaMemcpyAsync(ctx->d_occ + (size_t)min_x * gly, d_occ + (size_t)min_x * gly, (size_t)(max_x - min_x + 1) * gly,
@@ -280,12 +282,16 @@ int alore_esdf_last_sq(alore_ctx* ctx, int32_t* pos_sq, int32_t* neg_sq) {
   if (!pos_sq || !neg_sq) return alore_fail(ctx, ALORE_EINVAL, "null buffer");
   if (ctx->win[2] < ctx->win[0]) return alore_fail(ctx, ALORE_EINVAL, "no ESDF update has run on this context");
   ALORE_CUDA(ctx, cudaSetDevice(ctx->device));
+  // the last update may still run on a caller stream (alore_esdf_update_dev): its row pass is what is re-read here
+  ALORE_CUDA(ctx, cudaDeviceSynchronize());
   const int NX = ctx->win[2] - ctx->win[0] + 1, NY = ctx->win[3] - ctx->win[1] + 1;
   const size_t n = (size_t)NX * NY;
   int32_t *dp = nullptr, *dn = nullptr;
   ALORE_CUDA(ctx, cudaMalloc(&dp, n * sizeof(int32_t)));
   if (cudaMalloc(&dn, n * sizeof(int32_t)) != cudaSuccess) { cudaFree(dp); return alore_fail(ctx, ALORE_ENOMEM, "cudaMalloc"); }
-  int rc = alore_esdf_run(ctx, &ctx->geom, ctx->d_occ, ctx->d_dist, ctx->win[0], ctx->win[1], ctx->win[2], ctx->win[3],
+  // the window is checked against the grid the last update read: after a caller-buffer update that is the caller's
+  // geometry, not the resident map's (which may be absent or of another shape); the squared planes need no grid data
+  int rc = alore_esdf_run(ctx, &ctx->win_geom, ctx->d_occ, ctx->d_dist, ctx->win[0], ctx->win[1], ctx->win[2], ctx->win[3],
                           ctx->last_ref_compat, ctx->stream, dp, dn);
   if (rc == ALORE_OK) {
     cudaMemcpyAsync(pos_sq, dp, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream);

@@ -35,6 +35,7 @@ struct alore_ctx {
   int band_epoch = 0;            // flags of K2e are 'set' when they hold the current run's epoch
   int row_pitch = 0;
   int win[4] = {0, 0, -1, -1};   // min_x, min_y, max_x, max_y of the last update
+  alore_map_geom_t win_geom{};   // geometry of the grid the last update read (a caller buffer's, or the resident map's)
   int last_ref_compat = 1;
   float esdf_kernel_ms = 0.f;
   // host buffers page-locked through alore_host_register (lifetime guaranteed by the caller)

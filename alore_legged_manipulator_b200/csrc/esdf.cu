@@ -1179,7 +1179,9 @@ int alore_esdf_run(alore_ctx* ctx, const alore_map_geom_t* geom, const uint8_t* 
       if (ctx->d_band) { cudaDeviceSynchronize(); cudaFree(ctx->d_band); }
       ctx->d_band = nullptr; ctx->band_cap = 0;
       ALORE_CUDA(ctx, cudaMalloc(&ctx->d_band, need));
-      ALORE_CUDA(ctx, cudaMemset(ctx->d_band, 0, need));          // flags compare against a per-run epoch >= 1
+      // flags compare against a per-run epoch >= 1; zeroed on `st`, ahead of the K2 that reads them (a caller stream
+      // created non-blocking is not ordered after work on the legacy default stream)
+      ALORE_CUDA(ctx, cudaMemsetAsync(ctx->d_band, 0, need, st));
       ctx->band_cap = need;
       ctx->band_epoch = 0;
     }
@@ -1198,9 +1200,11 @@ int alore_esdf_run(alore_ctx* ctx, const alore_map_geom_t* geom, const uint8_t* 
       if (ctx->d_row) cudaFree(ctx->d_row);
       ctx->d_row = nullptr;
       ALORE_CUDA(ctx, cudaMalloc(&ctx->d_row, need_row * sizeof(int16_t)));
-      // columns NY..pitch-1 are never written by the row pass but travel through K2's 16-byte tile loads (no output
-      // depends on them): defined once, as "far from any seed"
-      ALORE_CUDA(ctx, cudaMemset(ctx->d_row, 0x7f, need_row * sizeof(int16_t)));
+      // columns NY..pitch-1 travel through K2's 16-byte tile loads but no output depends on them.  They are defined
+      // here once, as "far from any seed"; after that they hold whatever was last stored there: the fast row pass
+      // writes whole 16-cell groups (finite distances up to column 16*ceil(NY/16)-1), and an earlier, wider window of
+      // the same pitch leaves its own (also negative) values.  Zeroed on `st`, ahead of the row pass.
+      ALORE_CUDA(ctx, cudaMemsetAsync(ctx->d_row, 0x7f, need_row * sizeof(int16_t), st));
       ctx->row_cap = need_row;
     }
     if (need_blk > ctx->blk_cap) {
@@ -1211,6 +1215,7 @@ int alore_esdf_run(alore_ctx* ctx, const alore_map_geom_t* geom, const uint8_t* 
     }
     ctx->row_pitch = pitch;
     ctx->win[0] = min_x; ctx->win[1] = min_y; ctx->win[2] = max_x; ctx->win[3] = max_y;
+    ctx->win_geom = g;
     ctx->last_ref_compat = ref_compat;
     const size_t smem = (size_t)(((NY + 31 + 15) >> 4) << 4) + (size_t)NY * 2 + 16;
     if (smem > 48 * 1024)

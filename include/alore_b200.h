@@ -214,7 +214,9 @@ int alore_esdf_set(alore_ctx* ctx, const alore_map_geom_t* geom, const double* d
 
 /* Integer squared distances of the last alore_esdf_update[_dev] window (parity tests):
  * pos_sq/neg_sq host arrays of (max_x-min_x+1)*(max_y-min_y+1) int32, window-local index
- * x*NY + y; value ALORE_SQ_INF where the reference holds DBL_MAX. */
+ * x*NY + y; value ALORE_SQ_INF where the reference holds DBL_MAX.  Also after a caller-buffer
+ * alore_esdf_update_dev (then those buffers' planes, whatever the resident map is).  Waits for
+ * the device to be idle first, so a *_dev update still running on a caller stream is included. */
 #define ALORE_SQ_INF 0x7fffffff
 int alore_esdf_last_sq(alore_ctx* ctx, int32_t* pos_sq, int32_t* neg_sq);
 

@@ -46,7 +46,7 @@ def check_against_oracle(ctx, glx, gly, gi, grid, odom=(0.0, 0.0), rng_m=1e6, ch
 
 
 @pytest.mark.parametrize("shape", [(48, 40), (33, 57), (64, 64), (20, 90), (70, 25), (2, 2), (3, 5), (5, 3), (1, 7),
-                                   (200, 200), (130, 257), (257, 130)])
+                                   (200, 200), (130, 257), (257, 130), (24, 8193), (24, 16384)])
 @pytest.mark.parametrize("dens", [0.0, 1 / 400, 1 / 23, 1 / 3, 1.0])
 def test_small_maps_bit_exact(ctx, shape, dens):
     glx, gly = shape
