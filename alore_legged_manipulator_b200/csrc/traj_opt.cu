@@ -712,6 +712,15 @@ int alore_debug_force_exact_division(alore_ctx* ctx, int on) {
   return ALORE_OK;
 }
 
+int alore_debug_set_norm_guard(alore_ctx* ctx, double threshold) {
+  if (!ctx) return ALORE_EINVAL;
+  if (!(threshold > 0.0 && threshold <= 1e4)) return alore_fail(ctx, ALORE_EINVAL, "norm guard %g outside (0, 1e4]", threshold);
+  ALORE_CUDA(ctx, cudaSetDevice(ctx->device));
+  ALORE_CUDA(ctx, cudaDeviceSynchronize());
+  ALORE_CUDA(ctx, cudaMemcpyToSymbol(g_norm_guard, &threshold, sizeof(double)));
+  return ALORE_OK;
+}
+
 int alore_debug_phase_cycles(alore_ctx* ctx, unsigned long long* out32, int reset) {
   if (!ctx || !out32) return ALORE_EINVAL;
   ALORE_CUDA(ctx, cudaSetDevice(ctx->device));

@@ -1176,7 +1176,7 @@ __device__ __noinline__ bool step_candidate(const WParams& kp, const BatchDev& b
       s.skip = 0;
       if (s.phase != PH_FINAL) {
         const double ss = wdot(w.x, w.x, n, lane);
-        if (sqrt(ss) > 1e4) s.skip = 1;                      // costFunctionCallback returns `inf` (= 0) without touching g
+        if (sqrt(ss) > g_norm_guard) s.skip = 1;                      // costFunctionCallback returns `inf` (= 0) without touching g
         if (d_dirty) for (int i = lane; i < n; i += 32) dglob[i] = w.d[i];
       }
       break;
@@ -1249,7 +1249,7 @@ __global__ void wave_cost_prepare_kernel(const __grid_constant__ WParams kp, Bat
   const double ss = wdot(x, x, n, lane);
   if (lane == 0) {
     CandState s{};
-    s.phase = PH_INIT; s.stage = stage; s.skip = sqrt(ss) > 1e4 ? 1 : 0;
+    s.phase = PH_INIT; s.stage = stage; s.skip = sqrt(ss) > g_norm_guard ? 1 : 0;
     for (int d = 0; d < 2; d++) {
       s.lam[d] = lam ? lam[2 * b + d] : kp.P.EqualLambda[d];
       s.rho[d] = rho ? rho[2 * b + d] : kp.P.EqualRho[d];

@@ -321,8 +321,13 @@ int alore_selftest_division(alore_ctx* ctx, long long n_pairs, unsigned long lon
 /* Test hook: on != 0 makes every banded-solver pass use the compiler's division (the path taken when a quotient
  * leaves the split division's range); results must not change.  Process-wide for the context's device. */
 int alore_debug_force_exact_division(alore_ctx* ctx, int on);
+/* Test hook: the optimizer's cost evaluations return 0 without touching the gradient when ||x|| > threshold (the
+ * reference's `return inf;` with `#define inf 1 >> 30`, threshold 1e4 = the default).  A lower threshold makes that
+ * path reachable on ordinary candidates; threshold must lie in (0, 1e4].  Process-wide for the context's device. */
+int alore_debug_set_norm_guard(alore_ctx* ctx, double threshold);
 /* Developer hook: per-phase cycle totals of the optimizer kernels (only in builds with -DALORE_PHASE_TIMING;
- * the product build returns ALORE_EINVAL).  out32[0..6] = cost_eval phases, [8..13] = penalty passes, [16] = L-BFGS update. */
+ * the product build returns ALORE_EINVAL).  out32[0..6] = cost_eval phases ([4] penalty cost half, [7] penalty gradient half), [8..13] = penalty passes,
+ * [17..18] = L-BFGS update, [20] = history steps (a count), [21] = line-search trials whose gradient was skipped (a count). */
 int alore_debug_phase_cycles(alore_ctx* ctx, unsigned long long* out32, int reset);
 
 /* Developer hook: cycle / event counters of the wavefront optimizer's kernels (csrc/wave_opt.cuh g_wave_dbg): 16 values. */

@@ -75,8 +75,8 @@ else:
 import ctypes as C
 ph = (C.c_ulonglong * 32)()
 if ctx.lib.alore_debug_phase_cycles(ctx.h, ph, 1) == 0:
-    names = {0: "T-powers", 1: "LU+fwd", 2: "back", 3: "energy", 4: "penalty", 5: "adjoint", 6: "grad-out", 8: "  passA", 9: "  cells/prefix",
-             10: "  passB", 11: "  cost-sum", 12: "  fold", 13: "  passC", 17: "lbfgs s/y+dots", 18: "lbfgs two-loop", 20: "history steps (count, M)"}
-    tot = sum(ph[i] for i in (0, 1, 2, 3, 4, 5, 6, 17, 18))
+    names = {0: "T-powers", 1: "LU+fwd", 2: "back", 3: "energy", 4: "penalty cost", 7: "penalty grad", 5: "adjoint", 6: "grad-out", 8: "  passA", 9: "  cells/prefix",
+             10: "  passB", 11: "  cost-sum", 12: "  fold", 13: "  passC", 17: "lbfgs s/y+dots", 18: "lbfgs two-loop", 20: "history steps (count, M)", 21: "skipped grads (count, M)"}
+    tot = sum(ph[i] for i in (0, 1, 2, 3, 4, 5, 6, 7, 17, 18))
     for i, nme in names.items():
         print(f"phase {nme:16s} {ph[i]/1e6:12.1f} Mcycles  {100.0*ph[i]/max(tot,1):5.1f}%")
