@@ -313,7 +313,7 @@ EXPORTED_SYMBOLS = [
     "alore_esdf_last_kernel_ms", "alore_penalty_batch", "alore_penalty_batch_dev", "alore_cost_batch",
     "alore_opt_batch", "alore_batch_upload", "alore_batch_run", "alore_batch_download",
     "alore_batch_device_results", "alore_batch_argmin", "alore_batch_last_kernel_ms", "alore_batch_stats", "alore_batch_free",
-    "alore_final_collision_batch", "alore_selftest_division", "alore_debug_force_exact_division", "alore_debug_set_norm_guard", "alore_debug_phase_cycles", "alore_debug_wave_counters", "alore_launch_count",
+    "alore_final_collision_batch", "alore_selftest_division", "alore_debug_force_exact_division", "alore_debug_set_norm_guard", "alore_debug_phase_cycles", "alore_launch_count",
     "alore_create_multi", "alore_destroy_multi", "alore_multi_size", "alore_multi_ctx", "alore_multi_last_error",
     "alore_multi_esdf_update", "alore_multi_opt_batch",
 ]

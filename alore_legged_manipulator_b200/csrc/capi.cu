@@ -54,8 +54,6 @@ void alore_destroy(alore_ctx* ctx) {
   if (ctx->opt_scratch) cudaFree(ctx->opt_scratch);
   if (ctx->opt_hist) cudaFree(ctx->opt_hist);
   if (ctx->batch_pool) cudaFree(ctx->batch_pool);
-  if (ctx->h_poll) cudaFreeHost(ctx->h_poll);
-  for (auto& e : ctx->poll_ev) if (e) cudaEventDestroy(e);
   cudaEventDestroy(ctx->ev0);
   cudaEventDestroy(ctx->ev1);
   cudaEventDestroy(ctx->ev_fork);

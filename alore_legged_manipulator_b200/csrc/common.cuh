@@ -58,10 +58,7 @@ struct alore_ctx {
   std::vector<int32_t> sched_piece_off;
   std::vector<int32_t> sched_evals;
   void* last_batch = nullptr;                      // alore_batch of the last persistent-kernel run (its evals feed the next schedule)
-  // wavefront optimizer: pinned slots + events through which the host polls the survivor count (never per round)
   int l2_max_persist = -1, l2_max_window = -1;     // per device (set_l2_window)
-  int* h_poll = nullptr;
-  cudaEvent_t poll_ev[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
 };
 
 inline int alore_fail(alore_ctx* ctx, int code, const char* fmt, ...) {

@@ -7,7 +7,6 @@
 #include <numeric>
 
 #include "traj_opt.cuh"
-#include "wave_opt.cuh"
 
 using namespace topt;
 
@@ -263,6 +262,88 @@ collision_kernel(const __grid_constant__ KParams kp, int B, const int* piece_off
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// coefficient-space penalty kernel (alore_penalty_batch[_dev]): one 64-thread CTA per trajectory
+// ---------------------------------------------------------------------------------------------
+// scratch of the penalty passes (per resident CTA, stays in L2)
+struct PenLayout {
+  size_t cs, ax, ay, cellP, g2p, terms, nterm, rank, cg, fold, total;
+  int TS;
+  __host__ __device__ void init(int Nmax, int K, int KF, int ncp) {
+    const int Kbig = K > KF ? K : KF;
+    const size_t Smax = (size_t)Nmax * (2 * Kbig + 1);
+    size_t o = 0;
+    auto take = [&](size_t cnt) { size_t r = o; o += (cnt + 3) & ~size_t(3); return r; };
+    cs = take(2 * Smax); ax = take(Smax + 64); ay = take(Smax + 64);
+    cellP = take(2 * (size_t)Nmax * Kbig); g2p = take(2 * (size_t)Nmax * (Kbig + 1));
+    TS = (K + 1) * (7 + ncp) + 1;
+    terms = take((size_t)Nmax * TS); nterm = take(Nmax); rank = take((size_t)Nmax * (K + 1) + 32);
+    cg = take(2 * (size_t)Nmax * (K + 1)); fold = take(2 * (size_t)Nmax * (K + 1));
+    total = o;
+  }
+};
+
+struct PenParams {
+  alore_params_t P;
+  MapDev map;
+  PenLayout L;
+  int Nmax;
+};
+
+constexpr int PEN_NT = 64;   // threads per trajectory
+inline size_t pen_smem_doubles(int Nmax) {
+  // T1[N] gT[N] pXY[2(N+1)] bcast[4] | stg[1024] (cell-prefix chunks 2 x 256, cost-term packing 512)
+  return (size_t)Nmax + Nmax + 2 * (Nmax + 1) + 4 + 2 + 1024;
+}
+__device__ __forceinline__ void pen_carve(Warp& w, const PenLayout& L, double* smem, double* slab, int Nmax, int N, int K) {
+  w.lane = threadIdx.x;
+  w.N = N; w.n = 3 * N - 1; w.npad = (3 * N) & ~1; w.n6 = 6 * N; w.K = K; w.S1 = 2 * K + 1;
+  double* s = smem;
+  w.T1 = s; s += Nmax; w.gT = s; s += Nmax; w.pXY = s; s += 2 * (Nmax + 1); w.sumT = s; s += 4;
+  s = reinterpret_cast<double*>((reinterpret_cast<uintptr_t>(s) + 15) & ~uintptr_t(15));
+  w.stg = s;
+  w.Nm = Nmax;
+  w.cs = slab + L.cs; w.ax = slab + L.ax; w.ay = slab + L.ay; w.cellP = slab + L.cellP; w.g2p = slab + L.g2p;
+  w.terms = slab + L.terms; w.cg = slab + L.cg; w.fold = slab + L.fold;
+  w.nterm = reinterpret_cast<int*>(slab + L.nterm); w.rank = reinterpret_cast<int*>(slab + L.rank);
+  w.TS = L.TS;
+  w.err[0] = w.err[1] = 0.0;
+}
+
+// attachPenaltyFunctional on given coefficients (BASELINE configs[2]), one CTA per trajectory, reading the caller's
+// coefficient / duration arrays and accumulating straight into the caller's gradient arrays.
+__global__ void __launch_bounds__(PEN_NT, 6)
+penalty_cta_kernel(const __grid_constant__ PenParams kp, int B, const int* piece_off, const double* coeffs, const double* Ts,
+                   const double* start_xy, const double* final_xy, double* cost, double* gradC, double* gradT, double* err, double* slabs) {
+  extern __shared__ __align__(16) double smem[];
+  double* slab = slabs + (size_t)blockIdx.x * kp.L.total;
+  const int tid = threadIdx.x;
+#pragma unroll 1
+  for (int b = blockIdx.x; b < B; b += gridDim.x) {
+    const int p0 = piece_off[b], N = piece_off[b + 1] - p0;
+    if (N < 1 || N > kp.Nmax) {                               // more pieces than the caller declared: refuse, loudly (NaN), never overrun
+      if (tid == 0) { cost[b] = __longlong_as_double(0x7ff8000000000000ll); err[2 * b] = err[2 * b + 1] = 0.0; }
+      continue;
+    }
+    Warp w;
+    pen_carve(w, kp.L, smem, slab, kp.Nmax, N, kp.P.sparseResolution);
+    w.cf = const_cast<double*>(coeffs) + 12 * (size_t)p0;
+    w.gC = gradC + 12 * (size_t)p0;
+    w.sx = start_xy[2 * b]; w.sy = start_xy[2 * b + 1];
+    w.fx = final_xy[2 * b]; w.fy = final_xy[2 * b + 1];
+    for (int d = 0; d < 2; d++) { w.lam[d] = kp.P.EqualLambda[d]; w.rho[d] = kp.P.EqualRho[d]; }
+    w.safeDis = kp.P.safeDis;
+    w.init_pos = nullptr;
+    tsync<PEN_NT>();
+    for (int i = tid; i < 12 * N; i += PEN_NT) w.gC[i] = 0.0;
+    for (int i = tid; i < N; i += PEN_NT) { w.T1[i] = Ts[p0 + i]; w.gT[i] = 0.0; }
+    tsync<PEN_NT>();
+    const double f = penalty_passes_t<PEN_NT>(w, kp.P, kp.map, 1, 0.0);
+    for (int i = tid; i < N; i += PEN_NT) gradT[p0 + i] = w.gT[i];
+    if (tid == 0) { cost[b] = f; err[2 * b] = w.err[0]; err[2 * b + 1] = w.err[1]; }
+  }
+}
+
 // Lowest final cost among candidates with ok == 1 (ties -> lowest index).  One CTA.
 __global__ void argmin_kernel(int B, const double* cost, const int* ok, double* best_cost, int* best_idx) {
   __shared__ double sc[256];
@@ -451,216 +532,11 @@ struct alore_batch {
   std::vector<int32_t> piece_off;   // host copy (scheduling)
   int* d_order = nullptr;
   int runs = 0;
-  size_t* d_hist_off = nullptr;     // [B] offset (doubles) of each candidate's L-BFGS history ring, for mem_size = hist_m
-  int hist_m = 0;
-  size_t hist_doubles = 0;
   bool predicted = false;           // d_order currently holds a predicted (not piece-count) order
-  int rounds = 0;                   // rounds of the last run (one round = one cost evaluation of every unfinished candidate)
   bool pooled = false;              // device arrays carved from ctx->batch_pool
   char* pool_cur = nullptr;
   char* pool_end = nullptr;
 };
-
-// ---------------------------------------------------------------------------------------------
-// wavefront optimizer: host side (see wave_opt.cuh)
-// ---------------------------------------------------------------------------------------------
-namespace {
-
-struct WaveLaunch {
-  wave::WParams kp;
-  wave::WaveDev wd;
-  double* slabs = nullptr;
-  int grid_solve = 0, grid_pen = 0, grid_step = 0;
-  size_t smem_solve = 0, smem_pen = 0, smem_step = 0;
-};
-
-// Carves the per-candidate optimizer state of a batch with `tot` pieces from the context's scratch arena.
-int wave_prepare(alore_ctx* ctx, const alore_params_t* prm, int B, int tot, int Nmax, const int* d_piece_off, const size_t* d_hist_off,
-                 size_t hist_doubles, int mcap, WaveLaunch& L) {
-  if (!ctx->have_map || !ctx->d_dist) return alore_fail(ctx, ALORE_ENOMAP, "no ESDF resident on the device: call alore_esdf_update / alore_esdf_set first");
-  int rc = validate_opt_params(ctx, prm);
-  if (rc) return rc;
-  ALORE_CUDA(ctx, cudaSetDevice(ctx->device));
-  L.kp.P = *prm;
-  const alore_map_geom_t& g = ctx->geom;
-  L.kp.map = MapDev{ctx->d_dist, g.glx, g.gly, g.x_lower, g.y_lower, g.x_upper, g.y_upper, g.grid_interval, g.inv_grid_interval};
-  L.kp.L.init(Nmax, prm->sparseResolution, prm->finalSafeDisCheckNum, prm->n_checkpoints);
-  L.kp.Nmax = Nmax;
-  L.kp.npadmax = (3 * Nmax) & ~1;
-  L.kp.mcap = std::max(1, mcap);
-  L.smem_solve = (size_t)wave::SOLVE_WARPS * 4 * wave::GS * sizeof(double) + wave::GTAB * (sizeof(double) + sizeof(int));
-  L.smem_pen = wave::pen_smem_doubles(Nmax) * sizeof(double);
-  L.smem_step = wave::step_smem_doubles(Nmax) * sizeof(double);
-  if (L.smem_pen > 200 * 1024 || L.smem_step > 200 * 1024)
-    return alore_fail(ctx, ALORE_EINVAL, "trajectory with %d pieces exceeds the shared-memory budget", Nmax);
-  ALORE_CUDA(ctx, cudaFuncSetAttribute(wave::wave_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.smem_solve));
-  ALORE_CUDA(ctx, cudaFuncSetAttribute(wave::wave_adjoint_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.smem_solve));
-  ALORE_CUDA(ctx, cudaFuncSetAttribute(wave::wave_penalty_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.smem_pen));
-  ALORE_CUDA(ctx, cudaFuncSetAttribute(wave::wave_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.smem_step));
-  int occ_solve = 0, occ_pen = 0, occ_step = 0;
-  ALORE_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_solve, wave::wave_solve_kernel, 32 * wave::SOLVE_WARPS, L.smem_solve));
-  ALORE_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_pen, wave::wave_penalty_kernel, wave::PEN_NT, L.smem_pen));
-  ALORE_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_step, wave::wave_step_kernel, 32, L.smem_step));
-  if (occ_solve < 1 || occ_pen < 1 || occ_step < 1) return alore_fail(ctx, ALORE_EINVAL, "a round kernel does not fit on an SM");
-  const int per_cta = wave::SOLVE_WARPS * 4;
-  L.grid_solve = std::max(1, std::min((B + per_cta - 1) / per_cta, occ_solve * ctx->sm_count));
-  L.grid_pen = std::max(1, std::min(B, occ_pen * ctx->sm_count));
-  L.grid_step = std::max(1, std::min(B, std::min(occ_step, 16) * ctx->sm_count));
-
-  // arena: [state | lists | vectors | factors | slabs]
-  size_t o = 0;
-  auto take = [&](size_t bytes) { size_t r = o; o += (bytes + 255) & ~size_t(255); return r; };
-  const size_t o_cnt = take(2 * sizeof(int));
-  const size_t o_st = take((size_t)B * sizeof(wave::CandState));
-  const size_t o_l0 = take((size_t)B * sizeof(int)), o_l1 = take((size_t)B * sizeof(int));
-  const size_t v3 = 3 * (size_t)tot * sizeof(double), v1 = (size_t)tot * sizeof(double), v12 = 12 * (size_t)tot * sizeof(double),
-               v48 = 48 * (size_t)tot * sizeof(double);
-  const size_t o_x = take(v3), o_g = take(v3), o_xp = take(v3), o_gp = take(v3), o_d = take(v3);
-  const size_t o_T = take(v1), o_gT = take(v1);
-  const size_t o_cf = take(v12), o_gC = take(v12), o_zb = take(v12);
-  const size_t o_U = take(v48), o_L = take(v48);
-  const size_t o_pf = take(64 * (size_t)B * sizeof(double));
-  const size_t o_sl = take((size_t)std::max(L.grid_pen, L.grid_step) * L.kp.L.total * sizeof(double));
-  if (o > ctx->opt_scratch_bytes) {
-    if (ctx->opt_scratch) { cudaDeviceSynchronize(); cudaFree(ctx->opt_scratch); }
-    ctx->opt_scratch = nullptr; ctx->opt_scratch_bytes = 0;
-    ALORE_CUDA(ctx, cudaMalloc(&ctx->opt_scratch, o));
-    ctx->opt_scratch_bytes = o;
-  }
-  const size_t hbytes = std::max<size_t>(hist_doubles, 2) * sizeof(double);
-  if (hbytes > ctx->opt_hist_bytes) {
-    if (ctx->opt_hist) { cudaDeviceSynchronize(); cudaFree(ctx->opt_hist); }
-    ctx->opt_hist = nullptr; ctx->opt_hist_bytes = 0;
-    ALORE_CUDA(ctx, cudaMalloc(&ctx->opt_hist, hbytes));
-    ctx->opt_hist_bytes = hbytes;
-  }
-  char* base = static_cast<char*>(ctx->opt_scratch);
-  auto D = [&](size_t off) { return reinterpret_cast<double*>(base + off); };
-  wave::WaveDev& wd = L.wd;
-  wd.B = B; wd.m = L.kp.mcap;
-  wd.piece_off = d_piece_off; wd.hist_off = d_hist_off;
-  wd.x = D(o_x); wd.g = D(o_g); wd.xp = D(o_xp); wd.gp = D(o_gp); wd.d = D(o_d);
-  wd.T1 = D(o_T); wd.gT = D(o_gT); wd.cf = D(o_cf); wd.gC = D(o_gC); wd.zb = D(o_zb);
-  wd.Uf = D(o_U); wd.Lf = D(o_L); wd.pf = D(o_pf);
-  wd.hist = reinterpret_cast<double*>(ctx->opt_hist);
-  wd.st = reinterpret_cast<wave::CandState*>(base + o_st);
-  wd.list0 = reinterpret_cast<int*>(base + o_l0); wd.list1 = reinterpret_cast<int*>(base + o_l1);
-  wd.count = reinterpret_cast<int*>(base + o_cnt);
-  L.slabs = D(o_sl);
-  return ALORE_OK;
-}
-
-// Developer profile (env ALORE_WAVE_PROFILE=<csv path>): CUDA events around every kernel of every round.
-struct WaveProfile {
-  std::vector<cudaEvent_t> ev;
-  bool on = false;
-  void mark(cudaStream_t st) {
-    if (!on) return;
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    cudaEventRecord(e, st);
-    ev.push_back(e);
-  }
-};
-
-// the three evaluation kernels of a round for the survivor list `cur`
-void wave_eval_kernels(alore_ctx* ctx, const WaveLaunch& L, const BatchDev& bt, int cur, int known, cudaStream_t st, WaveProfile* pr = nullptr) {
-  const int per_cta = wave::SOLVE_WARPS * 4;
-  const int gs = std::max(1, std::min(L.grid_solve, (known + per_cta - 1) / per_cta));
-  const int gp = std::max(1, std::min(L.grid_pen, known));
-  if (pr) pr->mark(st);
-  wave::wave_solve_kernel<<<gs, 32 * wave::SOLVE_WARPS, L.smem_solve, st>>>(L.kp, bt, L.wd, cur);
-  if (pr) pr->mark(st);
-  wave::wave_penalty_kernel<<<gp, wave::PEN_NT, L.smem_pen, st>>>(L.kp, bt, L.wd, cur, L.slabs);
-  if (pr) pr->mark(st);
-  wave::wave_adjoint_kernel<<<gs, 32 * wave::SOLVE_WARPS, L.smem_solve, st>>>(L.kp, bt, L.wd, cur);
-  if (pr) pr->mark(st);
-  ctx->launches += 3;
-}
-
-__global__ void wave_list_init_kernel(int B, const int* order, int* list0, int* count) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < B) list0[i] = order ? order[i] : i;
-  if (i == 0) { count[0] = B; count[1] = 0; }
-}
-
-}  // namespace
-
-// B x MSPlanner::minco_plan as a wavefront (wave_opt.cuh).  Enqueues rounds on `st` and polls the survivor count with
-// a lag of two polls, so the device never waits for the host; returns when every candidate has finished.
-static int wave_run(alore_ctx* ctx, const alore_params_t* prm, alore_batch* bh, cudaStream_t st) {
-  const int B = bh->B;
-  const int mcap = std::max(1, std::max(prm->path_lbfgs.mem_size, prm->lbfgs.mem_size));
-  if (bh->hist_m != mcap || !bh->d_hist_off) {      // history ring offsets depend on mem_size
-    std::vector<size_t> ho(B);
-    size_t acc = 0;
-    for (int b = 0; b < B; b++) {
-      const size_t npad = (size_t)((3 * (bh->piece_off[b + 1] - bh->piece_off[b])) & ~1);
-      ho[b] = acc;
-      acc += (size_t)mcap * (2 * npad + 4);
-    }
-    if (!bh->d_hist_off) { ALORE_CUDA(ctx, cudaMalloc(&bh->d_hist_off, (size_t)B * sizeof(size_t))); bh->allocs.push_back(bh->d_hist_off); }
-    ALORE_CUDA(ctx, cudaMemcpyAsync(bh->d_hist_off, ho.data(), (size_t)B * sizeof(size_t), cudaMemcpyHostToDevice, st));
-    ALORE_CUDA(ctx, cudaStreamSynchronize(st));
-    bh->hist_m = mcap;
-    bh->hist_doubles = acc;
-  }
-  WaveLaunch L;
-  int rc = wave_prepare(ctx, prm, B, bh->tot, bh->Nmax, bh->bt.piece_off, bh->d_hist_off, bh->hist_doubles, mcap, L);
-  if (rc) return rc;
-  if (!ctx->h_poll) ALORE_CUDA(ctx, cudaHostAlloc(&ctx->h_poll, 64 * sizeof(int), cudaHostAllocDefault));
-  if (!ctx->poll_ev[0]) for (auto& e : ctx->poll_ev) ALORE_CUDA(ctx, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-  ALORE_CUDA(ctx, cudaEventRecord(bh->e0, st));
-  ALORE_CUDA(ctx, cudaMemsetAsync(L.wd.st, 0, (size_t)B * sizeof(wave::CandState), st));   // phase = PH_NEW
-  wave_list_init_kernel<<<(B + 255) / 256, 256, 0, st>>>(B, bh->bt.order, L.wd.list0, L.wd.count);
-  wave::wave_step_kernel<<<L.grid_step, 32, L.smem_step, st>>>(L.kp, bh->bt, bh->res, L.wd, 0, L.slabs);   // minco_plan prologue + x0
-  ctx->launches += 2;
-  int cur = 1, known = B, rounds = 0, polls = 0, chunk = 4;
-  bool done = false;
-  WaveProfile prof;
-  std::vector<int> prof_known;
-  prof.on = getenv("ALORE_WAVE_PROFILE") != nullptr;
-  while (!done) {
-    for (int r = 0; r < chunk; r++) {
-      wave_eval_kernels(ctx, L, bh->bt, cur, known, st, &prof);
-      wave::wave_step_kernel<<<std::max(1, std::min(L.grid_step, known)), 32, L.smem_step, st>>>(L.kp, bh->bt, bh->res, L.wd, cur, L.slabs);
-      prof.mark(st);
-      if (prof.on) prof_known.push_back(known);
-      ctx->launches++;
-      cur ^= 1;
-      rounds++;
-    }
-    ALORE_CUDA(ctx, cudaGetLastError());
-    // survivor count after this chunk -> pinned host slot, read two polls later
-    ALORE_CUDA(ctx, cudaMemcpyAsync(&ctx->h_poll[polls & 63], L.wd.count + cur, sizeof(int), cudaMemcpyDeviceToHost, st));
-    ALORE_CUDA(ctx, cudaEventRecord(ctx->poll_ev[polls & 7], st));
-    polls++;
-    if (polls >= 3) {
-      const int q = polls - 3;
-      ALORE_CUDA(ctx, cudaEventSynchronize(ctx->poll_ev[q & 7]));
-      known = ctx->h_poll[q & 63];
-      if (known == 0) done = true;
-    }
-    if (rounds > 4000000) return alore_fail(ctx, ALORE_ECUDA, "optimizer wavefront did not terminate");
-    chunk = known > 4096 ? 2 : 8;       // long rounds: poll often (the count shrinks the grids); short rounds: amortise the poll
-  }
-  ALORE_CUDA(ctx, cudaEventRecord(bh->e1, st));
-  bh->rounds = rounds;
-  if (prof.on) {
-    cudaStreamSynchronize(st);
-    if (FILE* fp = fopen(getenv("ALORE_WAVE_PROFILE"), "w")) {
-      fprintf(fp, "round,known,solve_ms,penalty_ms,adjoint_ms,step_ms\n");
-      for (size_t r = 0; r + 1 <= prof.ev.size() / 5; r++) {
-        float t[4];
-        for (int k = 0; k < 4; k++) cudaEventElapsedTime(&t[k], prof.ev[5 * r + k], prof.ev[5 * r + k + 1]);
-        fprintf(fp, "%zu,%d,%.5f,%.5f,%.5f,%.5f\n", r, prof_known[r], t[0], t[1], t[2], t[3]);
-      }
-      fclose(fp);
-    }
-    for (cudaEvent_t e : prof.ev) cudaEventDestroy(e);
-  }
-  return ALORE_OK;
-}
 
 // Longest-processing-time-first order.  Work estimate of a candidate = pieces x cost evaluations of the previous
 // optimisation of the same batch structure when known (replanning re-optimises nearly the same candidates every
@@ -734,15 +610,6 @@ int alore_debug_phase_cycles(alore_ctx* ctx, unsigned long long* out32, int rese
   std::memset(out32, 0, 32 * sizeof(unsigned long long));
   return alore_fail(ctx, ALORE_EINVAL, "library built without -DALORE_PHASE_TIMING");
 #endif
-}
-
-int alore_debug_wave_counters(alore_ctx* ctx, unsigned long long* out16, int reset) {
-  if (!ctx || !out16) return ALORE_EINVAL;
-  ALORE_CUDA(ctx, cudaSetDevice(ctx->device));
-  ALORE_CUDA(ctx, cudaDeviceSynchronize());
-  ALORE_CUDA(ctx, cudaMemcpyFromSymbol(out16, wave::g_wave_dbg, 16 * sizeof(unsigned long long)));
-  if (reset) { unsigned long long z[16] = {0}; ALORE_CUDA(ctx, cudaMemcpyToSymbol(wave::g_wave_dbg, z, sizeof(z))); }
-  return ALORE_OK;
 }
 
 int alore_selftest_division(alore_ctx* ctx, long long n_pairs, unsigned long long seed, long long* mismatches) {
@@ -829,66 +696,57 @@ int alore_batch_upload(alore_ctx* ctx, const alore_candidates_t* c, alore_batch*
 int alore_batch_run(alore_ctx* ctx, const alore_params_t* prm, alore_batch* bh, void* cuda_stream) {
   if (!ctx || !prm || !bh) return ALORE_EINVAL;
   cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
-  // Two implementations of the same computation, bit-identical results (scripts/opt_ab.py):
-  //  * persistent (default): one warp per candidate, asynchronous, longest-predicted-work first — faster whenever the
-  //    makespan is set by the heaviest candidate (it starts first and overlaps everything else);
-  //  * wavefront (ALORE_OPT_WAVE=1): lockstep rounds of small kernels (wave_opt.cuh) — fewer instructions in total and
-  //    independent of any schedule prediction, but every candidate advances at the pace of the round.
-  if (!getenv("ALORE_OPT_WAVE")) {
-    Launch L;
-    int rc = prepare_launch(ctx, prm, bh->Nmax, bh->B, opt_kernel, L, true);
-    if (rc) return rc;
-    // Hand-out order of the work queue: longest predicted work first.  Prediction = pieces x cost evaluations the
-    // candidate at the same index needed on the PREVIOUS tick (this handle's last run, or the last run of any handle
-    // on this context with the same structure: a replanning planner re-optimises mostly the same legs), else pieces.
-    if (ctx->last_batch) {                            // collect the previous tick's evaluation counts (it has finished: same-context ordering)
-      alore_batch* pb = static_cast<alore_batch*>(ctx->last_batch);
-      ALORE_CUDA(ctx, cudaEventSynchronize(pb->e1));   // that run may have been enqueued on another stream
-      std::vector<int32_t> ev(pb->B);
-      ALORE_CUDA(ctx, cudaMemcpyAsync(ev.data(), pb->res.evals, pb->B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  Launch L;
+  int rc = prepare_launch(ctx, prm, bh->Nmax, bh->B, opt_kernel, L, true);
+  if (rc) return rc;
+  // Hand-out order of the work queue: longest predicted work first.  Prediction = pieces x cost evaluations the
+  // candidate at the same index needed on the PREVIOUS tick (this handle's last run, or the last run of any handle
+  // on this context with the same structure: a replanning planner re-optimises mostly the same legs), else pieces.
+  if (ctx->last_batch) {                            // collect the previous tick's evaluation counts (it has finished: same-context ordering)
+    alore_batch* pb = static_cast<alore_batch*>(ctx->last_batch);
+    ALORE_CUDA(ctx, cudaEventSynchronize(pb->e1));   // that run may have been enqueued on another stream
+    std::vector<int32_t> ev(pb->B);
+    ALORE_CUDA(ctx, cudaMemcpyAsync(ev.data(), pb->res.evals, pb->B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    ALORE_CUDA(ctx, cudaStreamSynchronize(st));
+    ctx->sched_piece_off = pb->piece_off;
+    ctx->sched_evals.swap(ev);
+    ctx->last_batch = nullptr;
+  }
+  {
+    std::vector<int32_t> pred;
+    if (!getenv("ALORE_NO_SCHED_PREDICTION") && predicted_evals(ctx, bh->piece_off, pred)) {
+      std::vector<int> order;
+      lpt_order(bh->piece_off, pred.data(), order);
+      ALORE_CUDA(ctx, cudaMemcpyAsync(bh->d_order, order.data(), bh->B * sizeof(int), cudaMemcpyHostToDevice, st));
       ALORE_CUDA(ctx, cudaStreamSynchronize(st));
-      ctx->sched_piece_off = pb->piece_off;
-      ctx->sched_evals.swap(ev);
-      ctx->last_batch = nullptr;
+      bh->predicted = true;
+    } else if (bh->predicted) {                     // back to the piece-count order
+      std::vector<int> order;
+      lpt_order(bh->piece_off, nullptr, order);
+      ALORE_CUDA(ctx, cudaMemcpyAsync(bh->d_order, order.data(), bh->B * sizeof(int), cudaMemcpyHostToDevice, st));
+      ALORE_CUDA(ctx, cudaStreamSynchronize(st));
+      bh->predicted = false;
     }
-    {
-      std::vector<int32_t> pred;
-      if (!getenv("ALORE_NO_SCHED_PREDICTION") && predicted_evals(ctx, bh->piece_off, pred)) {
-        std::vector<int> order;
-        lpt_order(bh->piece_off, pred.data(), order);
-        ALORE_CUDA(ctx, cudaMemcpyAsync(bh->d_order, order.data(), bh->B * sizeof(int), cudaMemcpyHostToDevice, st));
-        ALORE_CUDA(ctx, cudaStreamSynchronize(st));
-        bh->predicted = true;
-      } else if (bh->predicted) {                     // back to the piece-count order
-        std::vector<int> order;
-        lpt_order(bh->piece_off, nullptr, order);
-        ALORE_CUDA(ctx, cudaMemcpyAsync(bh->d_order, order.data(), bh->B * sizeof(int), cudaMemcpyHostToDevice, st));
-        ALORE_CUDA(ctx, cudaStreamSynchronize(st));
-        bh->predicted = false;
-      }
-    }
-    bh->runs++;
-    ALORE_CUDA(ctx, cudaMemsetAsync(L.counter, 0, sizeof(int), st));
-    ALORE_CUDA(ctx, cudaEventRecord(bh->e0, st));
-    set_l2_window(ctx, st, L.slabs, (size_t)L.slots * L.kp.L.total * sizeof(double));
-    opt_kernel<<<L.slots, 32, L.smem, st>>>(L.kp, bh->bt, bh->res, L.slabs, L.hists, L.counter);
-    ctx->launches++;
-    clear_l2_window(st);
-    ALORE_CUDA(ctx, cudaGetLastError());
-    ALORE_CUDA(ctx, cudaEventRecord(bh->e1, st));
-    ctx->last_batch = bh;
-#ifdef ALORE_CAND_TIMING
-    if (const char* f = getenv("ALORE_CAND_TIMING_DUMP")) {
-      cudaDeviceSynchronize();
-      std::vector<unsigned long long> h(3 * 16384);
-      cudaMemcpyFromSymbol(h.data(), g_cand_ns, h.size() * sizeof(unsigned long long));
-      if (FILE* fp = fopen(f, "wb")) { fwrite(h.data(), sizeof(unsigned long long), h.size(), fp); fclose(fp); }
-    }
-#endif
-    return ALORE_OK;
   }
   bh->runs++;
-  return wave_run(ctx, prm, bh, st);
+  ALORE_CUDA(ctx, cudaMemsetAsync(L.counter, 0, sizeof(int), st));
+  ALORE_CUDA(ctx, cudaEventRecord(bh->e0, st));
+  set_l2_window(ctx, st, L.slabs, (size_t)L.slots * L.kp.L.total * sizeof(double));
+  opt_kernel<<<L.slots, 32, L.smem, st>>>(L.kp, bh->bt, bh->res, L.slabs, L.hists, L.counter);
+  ctx->launches++;
+  clear_l2_window(st);
+  ALORE_CUDA(ctx, cudaGetLastError());
+  ALORE_CUDA(ctx, cudaEventRecord(bh->e1, st));
+  ctx->last_batch = bh;
+#ifdef ALORE_CAND_TIMING
+  if (const char* f = getenv("ALORE_CAND_TIMING_DUMP")) {
+    cudaDeviceSynchronize();
+    std::vector<unsigned long long> h(3 * 16384);
+    cudaMemcpyFromSymbol(h.data(), g_cand_ns, h.size() * sizeof(unsigned long long));
+    if (FILE* fp = fopen(f, "wb")) { fwrite(h.data(), sizeof(unsigned long long), h.size(), fp); fclose(fp); }
+  }
+#endif
+  return ALORE_OK;
 }
 
 int alore_batch_download(alore_ctx* ctx, alore_batch* bh, alore_results_t* out) {
@@ -1013,21 +871,11 @@ int alore_cost_batch(alore_ctx* ctx, const alore_params_t* prm, const alore_cand
   if (safe_dis) { TRY(dev_copy(ctx, &d_sd, safe_dis, (size_t)B, st)) }
   TRY(dev_copy(ctx, &d_cost, (const double*)nullptr, (size_t)B, st))
   TRY(dev_copy(ctx, &d_err, (const double*)nullptr, 2 * (size_t)B, st))
-  if (getenv("ALORE_COST_PERSISTENT")) {
-    TRY(prepare_launch(ctx, prm, bh->Nmax, B, cost_kernel, L, false))
-    cudaMemsetAsync(L.counter, 0, sizeof(int), st);
-    cudaMemsetAsync(d_err, 0, 2 * (size_t)B * sizeof(double), st);
-    cost_kernel<<<L.slots, 32, L.smem, st>>>(L.kp, bh->bt, stage, d_x, d_lam, d_rho, d_sd, d_cost, d_g, d_err, L.slabs, L.counter);
-    ctx->launches++;
-  } else {
-    // one round of the wavefront's evaluation kernels at the caller's x
-    WaveLaunch W;
-    TRY(wave_prepare(ctx, prm, B, bh->tot, bh->Nmax, bh->bt.piece_off, nullptr, 0, 1, W))
-    wave::wave_cost_prepare_kernel<<<B, 32, 0, st>>>(W.kp, bh->bt, W.wd, stage, d_x, d_g, d_lam, d_rho, d_sd);
-    wave_eval_kernels(ctx, W, bh->bt, 0, B, st);
-    wave::wave_cost_finish_kernel<<<B, 32, 0, st>>>(W.kp, bh->bt, W.wd, d_cost, d_g, d_err);
-    ctx->launches += 2;
-  }
+  TRY(prepare_launch(ctx, prm, bh->Nmax, B, cost_kernel, L, false))
+  cudaMemsetAsync(L.counter, 0, sizeof(int), st);
+  cudaMemsetAsync(d_err, 0, 2 * (size_t)B * sizeof(double), st);
+  cost_kernel<<<L.slots, 32, L.smem, st>>>(L.kp, bh->bt, stage, d_x, d_lam, d_rho, d_sd, d_cost, d_g, d_err, L.slabs, L.counter);
+  ctx->launches++;
   cudaMemcpyAsync(cost, d_cost, (size_t)B * sizeof(double), cudaMemcpyDeviceToHost, st);
   cudaMemcpyAsync(g, d_g, nv * sizeof(double), cudaMemcpyDeviceToHost, st);
   if (xy_err) cudaMemcpyAsync(xy_err, d_err, 2 * (size_t)B * sizeof(double), cudaMemcpyDeviceToHost, st);
@@ -1048,49 +896,36 @@ static int penalty_launch(alore_ctx* ctx, const alore_params_t* prm, int B, int 
   if (rc) return rc;
   if (Nmax < 1) return alore_fail(ctx, ALORE_EINVAL, "max_pieces must be >= 1");
   ALORE_CUDA(ctx, cudaSetDevice(ctx->device));
-  wave::WParams kp;
+  PenParams kp;
   kp.P = *prm;
   const alore_map_geom_t& g = ctx->geom;
   kp.map = MapDev{ctx->d_dist, g.glx, g.gly, g.x_lower, g.y_lower, g.x_upper, g.y_upper, g.grid_interval, g.inv_grid_interval};
   kp.L.init(Nmax, prm->sparseResolution, prm->finalSafeDisCheckNum, prm->n_checkpoints);
-  kp.Nmax = Nmax; kp.npadmax = (3 * Nmax) & ~1; kp.mcap = 1;
-  // threads per trajectory x resident CTAs per SM x placement of the per-sample intermediates (tuning knob
-  // ALORE_PEN_SHAPE; default chosen by measurement on configs[2]: 64 threads, 6 CTAs per SM, intermediates in the L2-resident
-  // per-CTA slab — 0.65 ms; 128 threads 0.84, one warp 0.81, shared-memory intermediates 0.77 (8 warps per SM), more CTAs 0.69+,
-  // FEWER CTAs (ALORE_PEN_CTAS_PER_SM = 5 / 4 / 3) 0.71 / 0.80 / 0.98, a persisting-L2 window on the slabs 0.70: the 888 slabs
-  // of 160 KB exceed L2, but the kernel needs the parallelism more than the hit rate)
-  int shape = 64;
-  if (const char* e = getenv("ALORE_PEN_SHAPE")) shape = atoi(e);
-  const size_t smem_on = wave::pen_smem_doubles_onchip(Nmax, prm->sparseResolution) * sizeof(double);
-  const bool onchip = (shape == 641 || shape == 1281) && smem_on <= 200 * 1024;   // measured slower (0.77 vs 0.65 ms at configs[2]): opt-in
-  const size_t smem = onchip ? smem_on : wave::pen_smem_doubles(Nmax) * sizeof(double);
+  kp.Nmax = Nmax;
+  // 64 threads per trajectory, as many resident CTAs as fit (6 per SM), the per-sample intermediates in the per-CTA
+  // L2-resident slab: chosen by measurement on configs[2] (B200, DESIGN.md section 6): 0.65 ms; 128 threads 0.84, one
+  // warp 0.81, shared-memory intermediates 0.77 (8 warps per SM), more CTAs 0.69+, fewer CTAs (5 / 4 / 3 per SM)
+  // 0.71 / 0.80 / 0.98, a persisting-L2 window on the slabs 0.70: the 888 slabs of 160 KB exceed L2, but the kernel
+  // needs the parallelism more than the hit rate
+  const size_t smem = pen_smem_doubles(Nmax) * sizeof(double);
   if (smem > 200 * 1024) return alore_fail(ctx, ALORE_EINVAL, "trajectory with %d pieces exceeds the shared-memory budget", Nmax);
-  auto launch = [&](auto kern, int NT) -> int {
-    ALORE_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int occ = 0;
-    ALORE_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, NT, smem));
-    if (occ < 1) return alore_fail(ctx, ALORE_EINVAL, "kernel does not fit on an SM");
-    if (const char* e = getenv("ALORE_PEN_CTAS_PER_SM")) { const int v = atoi(e); if (v >= 1) occ = std::min(occ, v); }   // tuning knob
-    const int grid = std::max(1, std::min(B, occ * ctx->sm_count));
-    const size_t need = (size_t)grid * kp.L.total * sizeof(double);
-    if (need > ctx->opt_scratch_bytes) {
-      if (ctx->opt_scratch) { cudaDeviceSynchronize(); cudaFree(ctx->opt_scratch); }
-      ctx->opt_scratch = nullptr; ctx->opt_scratch_bytes = 0;
-      ALORE_CUDA(ctx, cudaMalloc(&ctx->opt_scratch, need));
-      ctx->opt_scratch_bytes = need;
-    }
-    kern<<<grid, NT, smem, st>>>(kp, B, d_piece_off, d_coeffs, d_piece_T, d_start_xy, d_final_xy, d_cost, d_gradC, d_gradT, d_xy_err,
-                                 reinterpret_cast<double*>(ctx->opt_scratch));
-    ctx->launches++;
-    ALORE_CUDA(ctx, cudaGetLastError());
-    return ALORE_OK;
-  };
-  if (shape == 32) return launch(wave::penalty_cta_kernel<32, 16, false>, 32);
-  if (shape == 128) return launch(wave::penalty_cta_kernel<128, 3, false>, 128);
-  if (shape == 640) return launch(wave::penalty_cta_kernel<64, 6, false>, 64);
-  if (shape == 1281 && onchip) return launch(wave::penalty_cta_kernel<128, 2, true>, 128);
-  if (onchip) return launch(wave::penalty_cta_kernel<64, 4, true>, 64);
-  return launch(wave::penalty_cta_kernel<64, 6, false>, 64);
+  ALORE_CUDA(ctx, cudaFuncSetAttribute(penalty_cta_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  int occ = 0;
+  ALORE_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, penalty_cta_kernel, PEN_NT, smem));
+  if (occ < 1) return alore_fail(ctx, ALORE_EINVAL, "kernel does not fit on an SM");
+  const int grid = std::max(1, std::min(B, occ * ctx->sm_count));
+  const size_t need = (size_t)grid * kp.L.total * sizeof(double);
+  if (need > ctx->opt_scratch_bytes) {
+    if (ctx->opt_scratch) { cudaDeviceSynchronize(); cudaFree(ctx->opt_scratch); }
+    ctx->opt_scratch = nullptr; ctx->opt_scratch_bytes = 0;
+    ALORE_CUDA(ctx, cudaMalloc(&ctx->opt_scratch, need));
+    ctx->opt_scratch_bytes = need;
+  }
+  penalty_cta_kernel<<<grid, PEN_NT, smem, st>>>(kp, B, d_piece_off, d_coeffs, d_piece_T, d_start_xy, d_final_xy, d_cost, d_gradC,
+                                                 d_gradT, d_xy_err, reinterpret_cast<double*>(ctx->opt_scratch));
+  ctx->launches++;
+  ALORE_CUDA(ctx, cudaGetLastError());
+  return ALORE_OK;
 }
 
 int alore_penalty_batch_dev(alore_ctx* ctx, const alore_params_t* prm, int B, int max_pieces, const int32_t* d_piece_off,

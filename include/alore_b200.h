@@ -330,9 +330,6 @@ int alore_debug_set_norm_guard(alore_ctx* ctx, double threshold);
  * [17..18] = L-BFGS update, [20] = history steps (a count), [21] = line-search trials whose gradient was skipped (a count). */
 int alore_debug_phase_cycles(alore_ctx* ctx, unsigned long long* out32, int reset);
 
-/* Developer hook: cycle / event counters of the wavefront optimizer's kernels (csrc/wave_opt.cuh g_wave_dbg): 16 values. */
-int alore_debug_wave_counters(alore_ctx* ctx, unsigned long long* out16, int reset);
-
 /* Number of kernels this library has launched since alore_create (bench `gpu_launches`). */
 long long alore_launch_count(const alore_ctx* ctx);
 

@@ -1,7 +1,6 @@
 """Sequential fuzz of minco_plan_batch on ONE context: random worlds (boxes), random leg batches (ragged piece counts,
-doglegs, cut trajectories), persistent and wavefront optimizer alternating, every result against the CPU oracle bit for
-bit (portable-trig contract).  usage: python scripts/opt_fuzz.py [rounds] [seed]"""
-import os, sys
+doglegs, cut trajectories), every result against the CPU oracle bit for bit (portable-trig contract).  usage: python scripts/opt_fuzz.py [rounds] [seed]"""
+import sys
 from pathlib import Path
 ROOT = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(ROOT)); sys.path.insert(0, str(ROOT / "tests"))
@@ -37,17 +36,13 @@ for it in range(rounds):
     pts = workloads.free_points(grid, m.geom(), m.distance_buffer_all_, int(rng.integers(5, 10)), int(rng.integers(1, 10**6)), min_clear=0.6)
     cands = workloads.leg_candidates(pts, headings=(0.0, float(rng.uniform(0.5, 3.0))), fe=fe, max_legs=int(rng.integers(20, 70)),
                                      dogleg=float(rng.uniform(0.0, 0.7)))
-    if it % 2:
-        os.environ["ALORE_OPT_WAVE"] = "1"
-    else:
-        os.environ.pop("ALORE_OPT_WAVE", None)
     res = pl.minco_plan_batch(cands)
     ref = oracle_lib.opt_batch(prm, m.geom(), m.distance_buffer_all_, cands, 8)
     worst = check_results(res, ref, cands)
     assert worst == 0.0, (it, worst)
     total += cands.B
     print(f"round {it}: {glx}x{gly}, {cands.B} candidates, pieces {int(np.diff(cands.piece_off).min())}..{int(np.diff(cands.piece_off).max())}, "
-          f"ok {int(res.ok.sum())}, replans max {int(res.replans.max())}, {'wave' if it % 2 else 'persistent'}: identical")
+          f"ok {int(res.ok.sum())}, replans max {int(res.replans.max())}: identical")
     m.close()
 olib.orc_set_trig_portable(0)
 print(f"opt fuzz: {rounds} rounds, {total} candidates ok (seed {seed})")

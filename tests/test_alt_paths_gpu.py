@@ -1,8 +1,9 @@
-"""The opt-in implementations must stay bit-identical to the default ones and to the oracle:
-  ALORE_OPT_WAVE=1    the lockstep wavefront optimizer (csrc/wave_opt.cuh) instead of the persistent kernel
+"""The opt-in ESDF implementations must stay bit-identical to the default ones and to the oracle:
   ALORE_ESDF_DC=1     the divide-and-conquer ESDF column pass instead of the register-window / expanding search
-  ALORE_PEN_SHAPE     threads per trajectory (and on-chip intermediates) of the coefficient-space penalty kernel
-The library reads these knobs at call time, so a test can flip them around a call."""
+  ALORE_ESDF_NO_BAND  the round-1 per-cell far search instead of the band lower-envelope kernel
+  ALORE_ESDF_SB       rows per band of the lower-envelope kernel (32/64/128/256)
+The library reads these knobs at call time, so a test can flip them around a call.  Also here: the device-pointer
+penalty entry, the coefficient-space penalty kernel against the oracle, and the reusable pinned result store."""
 import os
 from contextlib import contextmanager
 
@@ -10,10 +11,9 @@ import numpy as np
 import pytest
 
 import oracle_lib
-from alore_legged_manipulator_b200 import capi, front_end, workloads
-from alore_legged_manipulator_b200.ms_planner import MSPlanner
+from alore_legged_manipulator_b200 import capi, workloads
 from test_esdf_gpu import make_sdf
-from test_optimizer_gpu import check_results, leg_batch, portable_trig, world  # noqa: F401  (fixtures)
+from test_optimizer_gpu import leg_batch, portable_trig, world  # noqa: F401  (fixtures)
 
 pytestmark = pytest.mark.gpu
 
@@ -30,38 +30,6 @@ def env(**kw):
                 os.environ.pop(k, None)
             else:
                 os.environ[k] = v
-
-
-def test_wavefront_optimizer_bit_identical_to_persistent_and_oracle(world, portable_trig):
-    m, prm, pl, grid = world
-    cands = leg_batch(world, max_legs=96)
-    a = pl.minco_plan_batch(cands)                       # persistent kernel
-    with env(ALORE_OPT_WAVE=1):
-        b = pl.minco_plan_batch(cands)                   # wavefront
-    for f in ("ok", "status", "replans", "alm_iters", "evals", "cost", "coeffs", "piece_T", "inner_pts", "tail_s"):
-        assert np.array_equal(getattr(a, f), getattr(b, f)), f
-    ref = oracle_lib.opt_batch(prm, m.geom(), m.distance_buffer_all_, cands, 8)
-    assert check_results(b, ref, cands) == 0.0
-
-
-def test_wavefront_optimizer_replans_cut_and_long_trajectories(world, portable_trig, ctx):
-    """The resumable state machine through its rare transitions: collision replans (time_weight *= 0.75, restart from
-    get_state), failing candidates, the `if_cut` ALM parameter set; and N > 100 pieces (rolled two-loop fallback)."""
-    m, prm0, pl0, grid = world
-    prm = capi.default_params()
-    prm.alm_max_outer = 6
-    prm.finalMinSafeDis = 0.45
-    prm.safeReplanMaxTime = 2
-    pl = MSPlanner(ctx, prm, m)
-    fe = front_end.FrontEndParams()
-    fe.trajCutLength = 4.0
-    pts = workloads.free_points(grid, m.geom(), m.distance_buffer_all_, 7, 11, min_clear=0.5)
-    cands = workloads.leg_candidates(pts, headings=(0.0,), fe=fe, max_legs=40)
-    with env(ALORE_OPT_WAVE=1):
-        res = pl.minco_plan_batch(cands)
-    ref = oracle_lib.opt_batch(prm, m.geom(), m.distance_buffer_all_, cands, 8)
-    check_results(res, ref, cands)
-    assert res.replans.max() == 2 and (res.ok == 0).sum() > 0 and (res.ok == 1).sum() > 0
 
 
 @pytest.mark.parametrize("shape", [(257, 130), (64, 700), (1024, 1024)])
@@ -110,17 +78,12 @@ def test_esdf_far_field_paths_bit_exact(knobs):
     ctx.close()
 
 
-@pytest.mark.parametrize("shape", [32, 128, 640, 641, 1281])
-def test_penalty_kernel_shapes_bit_identical(world, portable_trig, shape):
+def test_penalty_kernel_bit_identical_to_oracle(world, portable_trig):
     m, prm, pl, grid = world
     po, coeffs, T, s_xy, f_xy = workloads.random_spline_batch(24, 40, m.geom(), m.distance_buffer_all_, grid, seed=5)
-    base = pl.penalty_batch(po, coeffs, T, s_xy, f_xy)
-    with env(ALORE_PEN_SHAPE=shape):
-        alt = pl.penalty_batch(po, coeffs, T, s_xy, f_xy)
-    for a, b in zip(base, alt):
-        assert np.array_equal(a, b)
-    cr, gCr, gTr, er = oracle_lib.penalty_batch(prm, m.geom(), m.distance_buffer_all_, po, coeffs, T, s_xy, f_xy, 4)
-    assert np.array_equal(alt[0], cr) and np.array_equal(alt[1], gCr) and np.array_equal(alt[2], gTr)
+    cost, gC, gT, _ = pl.penalty_batch(po, coeffs, T, s_xy, f_xy)
+    cr, gCr, gTr, _ = oracle_lib.penalty_batch(prm, m.geom(), m.distance_buffer_all_, po, coeffs, T, s_xy, f_xy, 4)
+    assert np.array_equal(cost, cr) and np.array_equal(gC, gCr) and np.array_equal(gT, gTr)
 
 
 def test_device_penalty_entry_refuses_undeclared_piece_counts(world, ctx):
