@@ -17,11 +17,11 @@ tail -n 3 "$OUT"/memcheck_r02.pytest.txt "$OUT"/racecheck_r02.pytest.txt
 grep -h "ERROR SUMMARY" "$OUT"/memcheck_r02.log "$OUT"/racecheck_r02.log
 # ESDF far-field path (K2 masks/flags, conditional K1b, K2e band envelope, warp-per-cell quirk column)
 compute-sanitizer --tool memcheck --error-exitcode 99 --log-file "$OUT"/memcheck_esdf_r02.log \
-  python -m pytest tests/test_esdf_gpu.py tests/test_alt_paths_gpu.py -x -q -m gpu -k "(small_maps or far_field or sub_window or named_maps) and not 4096 and not 8192" \
+  python -m pytest tests/test_esdf_gpu.py -x -q -m gpu -k "(small_maps or far_field or box_and_dense or sub_window or named_maps) and not 4096 and not 8192" \
   > "$OUT"/memcheck_esdf_r02.pytest.txt 2>&1
 echo "memcheck(esdf) rc=$?" >> "$OUT"/memcheck_esdf_r02.pytest.txt
 compute-sanitizer --tool racecheck --error-exitcode 99 --log-file "$OUT"/racecheck_esdf_r02.log \
-  python -m pytest tests/test_alt_paths_gpu.py -x -q -m gpu -k "far_field and (knobs0 or knobs2)" \
+  python -m pytest tests/test_esdf_gpu.py -x -q -m gpu -k "far_field_maps" \
   > "$OUT"/racecheck_esdf_r02.pytest.txt 2>&1
 echo "racecheck(esdf) rc=$?" >> "$OUT"/racecheck_esdf_r02.pytest.txt
 tail -n 3 "$OUT"/memcheck_esdf_r02.pytest.txt "$OUT"/racecheck_esdf_r02.pytest.txt

@@ -1,81 +1,13 @@
-"""The opt-in ESDF implementations must stay bit-identical to the default ones and to the oracle:
-  ALORE_ESDF_DC=1     the divide-and-conquer ESDF column pass instead of the register-window / expanding search
-  ALORE_ESDF_NO_BAND  the round-1 per-cell far search instead of the band lower-envelope kernel
-  ALORE_ESDF_SB       rows per band of the lower-envelope kernel (32/64/128/256)
-The library reads these knobs at call time, so a test can flip them around a call.  Also here: the device-pointer
-penalty entry, the coefficient-space penalty kernel against the oracle, and the reusable pinned result store."""
-import os
-from contextlib import contextmanager
-
+"""Entry points beside the main optimizer parity suite: the coefficient-space penalty kernel against the oracle, the
+device-pointer penalty entry and the reusable pinned result store."""
 import numpy as np
 import pytest
 
 import oracle_lib
 from alore_legged_manipulator_b200 import capi, workloads
-from test_esdf_gpu import make_sdf
 from test_optimizer_gpu import leg_batch, portable_trig, world  # noqa: F401  (fixtures)
 
 pytestmark = pytest.mark.gpu
-
-
-@contextmanager
-def env(**kw):
-    old = {k: os.environ.get(k) for k in kw}
-    os.environ.update({k: str(v) for k, v in kw.items()})
-    try:
-        yield
-    finally:
-        for k, v in old.items():
-            if v is None:
-                os.environ.pop(k, None)
-            else:
-                os.environ[k] = v
-
-
-@pytest.mark.parametrize("shape", [(257, 130), (64, 700), (1024, 1024)])
-def test_esdf_divide_and_conquer_column_pass_bit_exact(shape):
-    import alore_legged_manipulator_b200 as alore
-    ctx = alore.Context(0)                # its own context: one context holds one device-resident map
-    glx, gly = shape
-    for seed, kw in ((1, dict(p_occ=0.02, p_unknown=0.01)), (2, dict(p_occ=0.0, p_unknown=0.0, boxes=6, box_cells=(4, 40))),
-                     (3, dict(p_occ=0.7, p_unknown=0.05))):
-        grid = workloads.random_map(glx, gly, seed, **kw)
-        m = make_sdf(ctx, glx, gly, 0.05, grid)
-        with env(ALORE_ESDF_DC=1):
-            m.updateESDF2d()
-        ref = np.full(glx * gly, np.finfo(np.float64).max)
-        mn, mx = m.esdf_window()
-        oracle_lib.esdf_update(m.geom(), grid, mn, mx, ref)
-        assert np.array_equal(m.distance_buffer_all_.view(np.uint64), ref.view(np.uint64)), (shape, seed)
-        m.close()
-    ctx.close()
-
-
-@pytest.mark.parametrize("knobs", [dict(ALORE_ESDF_NO_BAND=1), dict(ALORE_ESDF_SB=32), dict(ALORE_ESDF_SB=64),
-                                   dict(ALORE_ESDF_SB=128), dict(ALORE_ESDF_SB=256)])
-def test_esdf_far_field_paths_bit_exact(knobs):
-    """Far cells (large empty / solid regions): the band lower-envelope kernel at every band height and the round-1
-    per-cell search must all reproduce the oracle bit for bit, on maps that are nearly empty, nearly solid and mixed."""
-    import alore_legged_manipulator_b200 as alore
-    ctx = alore.Context(0)
-    for (glx, gly), seed, kw in (((700, 300), 2, dict(p_occ=0.0, p_unknown=0.0, boxes=5, box_cells=(4, 40))),
-                                 ((513, 257), 3, dict(p_occ=0.0, p_unknown=0.0, wall=False, boxes=1, box_cells=(2, 3))),
-                                 ((300, 900), 4, dict(p_occ=0.0, p_unknown=0.0, boxes=30, box_cells=(40, 200))),
-                                 ((1100, 260), 5, dict(p_occ=1.0, p_unknown=0.0))):
-        grid = workloads.random_map(glx, gly, seed, **kw)
-        if kw.get("p_occ") == 1.0:                           # a solid world with one free pocket and one free cell
-            g2 = grid.reshape(glx, gly)
-            g2[500:520, 100:130] = workloads.UNOCCUPIED
-            g2[40, 200] = workloads.UNOCCUPIED
-        m = make_sdf(ctx, glx, gly, 0.05, grid)
-        with env(**knobs):
-            m.updateESDF2d()
-        ref = np.full(glx * gly, np.finfo(np.float64).max)
-        mn, mx = m.esdf_window()
-        oracle_lib.esdf_update(m.geom(), grid, mn, mx, ref)
-        assert np.array_equal(m.distance_buffer_all_.view(np.uint64), ref.view(np.uint64)), ((glx, gly), seed, knobs)
-        m.close()
-    ctx.close()
 
 
 def test_penalty_kernel_bit_identical_to_oracle(world, portable_trig):

@@ -14,8 +14,7 @@ from scipy import ndimage
 
 import oracle_lib
 from alore_legged_manipulator_b200 import capi, workloads
-from test_alt_paths_gpu import env
-from test_esdf_gpu import patchwork_map
+from test_esdf_gpu import far_field_maps as far_field_grids, patchwork_map
 from test_esdf_oracle import SHAPES, brute_force_expected
 from test_optimizer_gpu import check_results, portable_trig  # noqa: F401  (fixture)
 
@@ -264,19 +263,8 @@ def check_clean(ctx, geom, occ, mn, mx, sq=True, host=True, occ_offset=0):
 
 # ---- maps --------------------------------------------------------------------------------------------------------
 def far_field_maps():
-    """The four maps of test_alt_paths_gpu.test_esdf_far_field_paths_bit_exact (nearly empty, nearly solid, mixed)."""
-    out = []
-    for (glx, gly), seed, kw in (((700, 300), 2, dict(p_occ=0.0, p_unknown=0.0, boxes=5, box_cells=(4, 40))),
-                                 ((513, 257), 3, dict(p_occ=0.0, p_unknown=0.0, wall=False, boxes=1, box_cells=(2, 3))),
-                                 ((300, 900), 4, dict(p_occ=0.0, p_unknown=0.0, boxes=30, box_cells=(40, 200))),
-                                 ((1100, 260), 5, dict(p_occ=1.0, p_unknown=0.0))):
-        grid = workloads.random_map(glx, gly, seed, **kw)
-        if kw.get("p_occ") == 1.0:
-            g2 = grid.reshape(glx, gly)
-            g2[500:520, 100:130] = FREE
-            g2[40, 200] = FREE
-        out.append((glx, gly, grid, (0, 0), (glx - 1, gly - 1)))
-    return out
+    """The four maps of test_esdf_gpu.test_far_field_maps_bit_exact (nearly empty, nearly solid, mixed), whole windows."""
+    return [(glx, gly, grid, (0, 0), (glx - 1, gly - 1)) for glx, gly, grid in far_field_grids()]
 
 
 def patchwork_windows(n, seed0=500):
@@ -308,20 +296,15 @@ def degenerate_windows():
     return [(glx, gly, grid, mn, mx) for mn, mx in wins]
 
 
-KNOBS = [dict(), dict(ALORE_ESDF_NO_BAND=1), dict(ALORE_ESDF_SB=256), dict(ALORE_ESDF_DC=1)]
-
-
 @gpu
-@pytest.mark.parametrize("knobs", KNOBS, ids=["default", "no_band", "sb256", "dc"])
-def test_device_write_set_equals_reference_write_set(knobs):
+def test_device_write_set_equals_reference_write_set():
     """ref_compat: the device buffer holds exactly the reference's writes (window minus its last row and column);
     every other cell keeps its sentinel.  The largest map also checks both squared planes of the caller-buffer update."""
     ctx = new_ctx()
     cases = patchwork_windows(6) + far_field_maps() + uniform_maps() + degenerate_windows()
     largest = max(range(len(cases)), key=lambda i: (cases[i][4][0] - cases[i][3][0] + 1) * (cases[i][4][1] - cases[i][3][1] + 1))
-    with env(**knobs):
-        for i, (glx, gly, grid, mn, mx) in enumerate(cases):
-            check_ref_compat(ctx, workloads.make_geom(glx, gly, 0.05), grid, mn, mx, sq=(i == largest))
+    for i, (glx, gly, grid, mn, mx) in enumerate(cases):
+        check_ref_compat(ctx, workloads.make_geom(glx, gly, 0.05), grid, mn, mx, sq=(i == largest))
     ctx.close()
 
 
@@ -360,14 +343,12 @@ def test_clean_mode_corridor_8192x2048_exact():
 
 
 @gpu
-@pytest.mark.parametrize("knobs", KNOBS[:2], ids=["default", "no_band"])
-def test_clean_mode_far_field_patchwork_and_uniform_exact(knobs):
-    """Far cells in clean mode (the band kernel and the pruned search), windows anywhere, all-free and all-Occupied
-    windows (gi*sqrt(DBL_MAX) for the missing kind), degenerate windows."""
+def test_clean_mode_far_field_patchwork_and_uniform_exact():
+    """Far cells in clean mode (the band kernel), windows anywhere, all-free and all-Occupied windows
+    (gi*sqrt(DBL_MAX) for the missing kind), degenerate windows."""
     ctx = new_ctx()
-    with env(**knobs):
-        for glx, gly, grid, mn, mx in far_field_maps() + patchwork_windows(8, 900) + uniform_maps() + degenerate_windows():
-            check_clean(ctx, workloads.make_geom(glx, gly, 0.05), grid, mn, mx)
+    for glx, gly, grid, mn, mx in far_field_maps() + patchwork_windows(8, 900) + uniform_maps() + degenerate_windows():
+        check_clean(ctx, workloads.make_geom(glx, gly, 0.05), grid, mn, mx)
     ctx.close()
 
 
@@ -446,22 +427,20 @@ def corner_strip(NX, NY, inverted):
 
 
 @gpu
-@pytest.mark.parametrize("knobs", KNOBS[:2], ids=["default", "no_band"])
 @pytest.mark.parametrize("shape", [(16384, 48), (48, 16384)])
-def test_window_limit_corner_seed_strips(shape, knobs):
-    """16384-cell sides: far cells everywhere (band kernel), the aliased column over 16384 rows, and with
-    ALORE_ESDF_NO_BAND on 16384 rows the super-block minima (512 blocks > 128)."""
+def test_window_limit_corner_seed_strips(shape):
+    """16384-cell sides: far cells everywhere (band kernel, 512 blocks of minima per column on 16384 rows) and the
+    aliased column over 16384 rows."""
     NX, NY = shape
     ctx = new_ctx()
     geom = workloads.make_geom(NX, NY, 0.05)
-    with env(**knobs):
-        for inverted in (False, True):
-            grid = corner_strip(NX, NY, inverted)
-            check_ref_compat(ctx, geom, grid, (0, 0), (NX - 1, NY - 1), sq=True)
-            check_clean(ctx, geom, grid, (0, 0), (NX - 1, NY - 1), host=False)
-            pos, neg = last_sq(ctx, (0, 0), (NX - 1, NY - 1))
-            plane = neg if inverted else pos
-            assert plane.max() == (NX - 1) ** 2 + (NY - 1) ** 2        # the far corner, exactly
+    for inverted in (False, True):
+        grid = corner_strip(NX, NY, inverted)
+        check_ref_compat(ctx, geom, grid, (0, 0), (NX - 1, NY - 1), sq=True)
+        check_clean(ctx, geom, grid, (0, 0), (NX - 1, NY - 1), host=False)
+        pos, neg = last_sq(ctx, (0, 0), (NX - 1, NY - 1))
+        plane = neg if inverted else pos
+        assert plane.max() == (NX - 1) ** 2 + (NY - 1) ** 2        # the far corner, exactly
     ctx.close()
 
 

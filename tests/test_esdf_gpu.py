@@ -123,6 +123,56 @@ def test_config5_shape_8192x2048_bit_exact(ctx):
     check_against_oracle(ctx, glx, gly, 0.005, grid, check_sq=False)
 
 
+@pytest.mark.parametrize("shape", [(257, 130), (64, 700), (1024, 1024)])
+def test_sparse_box_and_dense_maps_bit_exact(shape):
+    """Sparse clutter, a box world and a dense map of each shape, on a context of their own."""
+    import alore_legged_manipulator_b200 as alore
+    ctx = alore.Context(0)                # its own context: one context holds one device-resident map
+    glx, gly = shape
+    for seed, kw in ((1, dict(p_occ=0.02, p_unknown=0.01)), (2, dict(p_occ=0.0, p_unknown=0.0, boxes=6, box_cells=(4, 40))),
+                     (3, dict(p_occ=0.7, p_unknown=0.05))):
+        grid = workloads.random_map(glx, gly, seed, **kw)
+        m = make_sdf(ctx, glx, gly, 0.05, grid)
+        m.updateESDF2d()
+        ref = np.full(glx * gly, DBL_MAX)
+        mn, mx = m.esdf_window()
+        oracle_lib.esdf_update(m.geom(), grid, mn, mx, ref)
+        assert np.array_equal(m.distance_buffer_all_.view(np.uint64), ref.view(np.uint64)), (shape, seed)
+        m.close()
+    ctx.close()
+
+
+def far_field_maps():
+    """(glx, gly, grid): nearly empty, nearly solid and mixed maps, where most cells are left to the band kernel."""
+    out = []
+    for (glx, gly), seed, kw in (((700, 300), 2, dict(p_occ=0.0, p_unknown=0.0, boxes=5, box_cells=(4, 40))),
+                                 ((513, 257), 3, dict(p_occ=0.0, p_unknown=0.0, wall=False, boxes=1, box_cells=(2, 3))),
+                                 ((300, 900), 4, dict(p_occ=0.0, p_unknown=0.0, boxes=30, box_cells=(40, 200))),
+                                 ((1100, 260), 5, dict(p_occ=1.0, p_unknown=0.0))):
+        grid = workloads.random_map(glx, gly, seed, **kw)
+        if kw.get("p_occ") == 1.0:                           # a solid world with one free pocket and one free cell
+            g2 = grid.reshape(glx, gly)
+            g2[500:520, 100:130] = capi.UNOCCUPIED
+            g2[40, 200] = capi.UNOCCUPIED
+        out.append((glx, gly, grid))
+    return out
+
+
+def test_far_field_maps_bit_exact():
+    """Far cells (large empty / solid regions) must reproduce the oracle bit for bit."""
+    import alore_legged_manipulator_b200 as alore
+    ctx = alore.Context(0)
+    for glx, gly, grid in far_field_maps():
+        m = make_sdf(ctx, glx, gly, 0.05, grid)
+        m.updateESDF2d()
+        ref = np.full(glx * gly, DBL_MAX)
+        mn, mx = m.esdf_window()
+        oracle_lib.esdf_update(m.geom(), grid, mn, mx, ref)
+        assert np.array_equal(m.distance_buffer_all_.view(np.uint64), ref.view(np.uint64)), (glx, gly)
+        m.close()
+    ctx.close()
+
+
 def patchwork_map(glx, gly, rng):
     """Rectangles of very different character side by side: solid, empty, cluttered, sparse seeds, unknown."""
     g = np.full((glx, gly), capi.UNOCCUPIED, dtype=np.uint8)
