@@ -89,6 +89,29 @@ class Results(C.Structure):
     ]
 
 
+class Task(C.Structure):
+    """alore_task_t: task points 0 robot, 1..n objects, n+1..2n targets; leg labels of the candidates."""
+
+    _fields_ = [
+        ("n_objects", C.c_int32), ("fixed_assignment", C.c_int32), ("assign", c_int32_p),
+        ("leg_from", c_int32_p), ("leg_to", c_int32_p),
+    ]
+
+
+class TaskPlanOut(C.Structure):
+    """alore_task_plan_t: the optimum, the plan, and (optional) the leg matrix."""
+
+    _fields_ = [
+        ("cost", C.c_double), ("feasible", C.c_int32), ("reserved", C.c_int32),
+        ("order", c_int32_p), ("target", c_int32_p), ("leg_cand", c_int32_p),
+        ("leg_cost", c_double_p), ("leg_best", c_int32_p),
+    ]
+
+
+ALORE_TASK_MAX_FREE = 12
+ALORE_TASK_MAX_FIXED = 20
+
+
 def dptr(a: np.ndarray):
     assert a.dtype == np.float64 and a.flags["C_CONTIGUOUS"]
     return a.ctypes.data_as(c_double_p)
@@ -300,6 +323,8 @@ def load_library(path: os.PathLike | None = None) -> C.CDLL:
         lib.alore_debug_set_norm_guard.argtypes = [vp, C.c_double]
         lib.alore_debug_phase_cycles.argtypes = [vp, C.POINTER(C.c_ulonglong), C.c_int]
         lib.alore_selftest_division.argtypes = [vp, C.c_longlong, C.c_ulonglong, C.POINTER(C.c_longlong)]
+        lib.alore_task_plan.argtypes = [vp, C.POINTER(Task), C.c_int, c_double_p, c_int32_p, C.POINTER(TaskPlanOut)]
+        lib.alore_batch_task_plan.argtypes = [vp, vp, C.POINTER(Task), C.POINTER(TaskPlanOut)]
     if path is None:
         _lib = lib
     return lib
@@ -315,7 +340,7 @@ EXPORTED_SYMBOLS = [
     "alore_batch_device_results", "alore_batch_argmin", "alore_batch_last_kernel_ms", "alore_batch_stats", "alore_batch_free",
     "alore_final_collision_batch", "alore_selftest_division", "alore_debug_force_exact_division", "alore_debug_set_norm_guard", "alore_debug_phase_cycles", "alore_launch_count",
     "alore_create_multi", "alore_destroy_multi", "alore_multi_size", "alore_multi_ctx", "alore_multi_last_error",
-    "alore_multi_esdf_update", "alore_multi_opt_batch",
+    "alore_multi_esdf_update", "alore_multi_opt_batch", "alore_task_plan", "alore_batch_task_plan",
 ]
 
 

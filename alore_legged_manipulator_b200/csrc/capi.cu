@@ -54,6 +54,7 @@ void alore_destroy(alore_ctx* ctx) {
   if (ctx->opt_scratch) cudaFree(ctx->opt_scratch);
   if (ctx->opt_hist) cudaFree(ctx->opt_hist);
   if (ctx->batch_pool) cudaFree(ctx->batch_pool);
+  if (ctx->task_pool) cudaFree(ctx->task_pool);
   cudaEventDestroy(ctx->ev0);
   cudaEventDestroy(ctx->ev1);
   cudaEventDestroy(ctx->ev_fork);

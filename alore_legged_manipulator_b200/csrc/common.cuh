@@ -59,6 +59,10 @@ struct alore_ctx {
   std::vector<int32_t> sched_evals;
   void* last_batch = nullptr;                      // alore_batch of the last persistent-kernel run (its evals feed the next schedule)
   int l2_max_persist = -1, l2_max_window = -1;     // per device (set_l2_window)
+
+  // ---- task plan scratch (see task.cu): leg matrix, DP layers, plan; grown on demand, reused across calls ----
+  void* task_pool = nullptr;
+  size_t task_pool_bytes = 0;
 };
 
 inline int alore_fail(alore_ctx* ctx, int code, const char* fmt, ...) {
@@ -84,3 +88,5 @@ int alore_esdf_run(alore_ctx* ctx, const alore_map_geom_t* geom, const uint8_t* 
 // capi.cu: alore_esdf_update with an optional host mirror (dist_inout == NULL: keep the result in HBM only)
 int alore_esdf_update_impl(alore_ctx* ctx, const alore_map_geom_t* geom, const uint8_t* occ, int min_x, int min_y, int max_x,
                            int max_y, double* dist_inout, int ref_compat);
+// traj_opt.cu: size, run count and device cost/ok arrays of a batch handle (for task.cu)
+void batch_result_view(const alore_batch* bh, int* B, int* runs, const double** d_cost, const int32_t** d_ok);

@@ -538,6 +538,13 @@ struct alore_batch {
   char* pool_end = nullptr;
 };
 
+void batch_result_view(const alore_batch* bh, int* B, int* runs, const double** d_cost, const int32_t** d_ok) {
+  *B = bh->B;
+  *runs = bh->runs;
+  *d_cost = bh->res.cost;
+  *d_ok = bh->res.ok;
+}
+
 // Longest-processing-time-first order.  Work estimate of a candidate = pieces x cost evaluations of the previous
 // optimisation of the same batch structure when known (replanning re-optimises nearly the same candidates every
 // tick), else pieces alone.  Only the hand-out order of the work queue changes, never a result.

@@ -40,6 +40,16 @@ class DeviceBatch:
         self.ctx.check(self.ctx.lib.alore_batch_argmin(self.ctx.h, self.h, C.byref(bc), C.byref(bi)))
         return float(bc.value), int(bi.value)
 
+    def task_plan(self, n_objects, leg_from, leg_to, fixed_assignment=False, assign=None, with_matrix=False):
+        """alore_batch_task_plan: the task plan (task_planner.TaskPlan) from the device results of the last run, one
+        leg label per candidate of this batch."""
+        from .task_planner import TaskCall
+        call = TaskCall(n_objects, leg_from, leg_to, fixed_assignment, assign, with_matrix)
+        if call.B != self.cands.B:
+            raise ValueError(f"{call.B} leg labels for a batch of {self.cands.B} candidates")
+        self.ctx.check(self.ctx.lib.alore_batch_task_plan(self.ctx.h, self.h, C.byref(call.task), C.byref(call.out)))
+        return call.result()
+
     def device_results(self):
         dc, dk = C.c_void_p(), C.c_void_p()
         self.ctx.check(self.ctx.lib.alore_batch_device_results(self.h, C.byref(dc), C.byref(dk)))

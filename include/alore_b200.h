@@ -295,6 +295,59 @@ int alore_final_collision_batch(alore_ctx* ctx, const alore_params_t* prm, int B
                                 const double* piece_T, const double* start_xy,
                                 int32_t* collided, double* min_dist);
 
+/* ---- task plan: leg cost matrix of the optimised candidates + exact visiting order x assignment search -------------
+ * Task points: 0 = the robot, 1..n = the objects, n+1..2n = the targets, P = 2n+1.  The caller labels every candidate b
+ * with the leg it belongs to, leg_from[b] -> leg_to[b] in [0, P), from != to; leg_from[b] = -1 marks a candidate that
+ * is not a task leg (ignored), so a batch may hold other candidates too.
+ *
+ * Leg matrix D[P][P]: a candidate counts when ok[b] == 1 and cost[b] is finite.  best[i][j] = the lowest candidate index
+ * among the counted candidates of leg (i, j) whose cost compares equal (IEEE ==) to their minimum; D[i][j] =
+ * cost[best[i][j]] with its exact bits.  A leg without a counted candidate has D = +inf and best = -1.  The minimum over
+ * heading variants is part of this contract; heading continuity between consecutive legs is not modelled.
+ *
+ * Tour: objects picked in the order o_1..o_n, o_k carried to target t_k (a bijection onto the targets), starting at the
+ * robot and ending at the last target (no return).  Legs in tour order: 0->o_1, o_1->t_1, t_1->o_2, ..., o_n->t_n.  Its
+ * cost is the left fold in tour order, c = D[0][o_1], then c = c + D[next leg], each addition rounded in IEEE double.
+ * fixed_assignment = 1: t_k = assign[o_k - 1] (assign NULL: object i -> target n+i); only the order is searched.
+ * fixed_assignment = 0: order and assignment are searched jointly.
+ *
+ * Exact layered DP over O (objects picked so far) and T (targets filled so far):
+ *   A[O,T,j] (|O| = |T|+1, j in O just picked) = D[0][j] for T empty, else min over t in T of B[O\{j},T,t] + D[t][j]
+ *   B[O,T,u] (|O| = |T|, u in T just filled)   = min over j in O of A[O,T\{u},j] + D[j][u]  (fixed: only u = assign(j))
+ * optimum = min over u of B[all,all,u] (fixed mode: over j, u = assign(j)).  Since x -> fl(x + a) is monotone, this is
+ * exactly the minimum of the fold over all tours, bit for bit.  Tie rule: every minimum scans its candidates in
+ * ascending point index and replaces only on strict <; the plan is the backtrack of these choices.  Negative costs are
+ * allowed.  The plan is feasible iff the optimum is < +inf; otherwise order, target and leg_cand are -1.
+ * Limits: n <= ALORE_TASK_MAX_FREE (about 16.2 M states per half-step, ~290 MB of device scratch) in free mode,
+ * n <= ALORE_TASK_MAX_FIXED (10.5 M states per half-step, ~190 MB) in fixed mode; larger n returns ALORE_EINVAL.
+ * Inputs are validated on the host before any launch (ALORE_EINVAL with a message; the context stays usable).  Device
+ * scratch is an arena of the context that grows on demand.  Both entry points are blocking. */
+#define ALORE_TASK_MAX_FREE 12
+#define ALORE_TASK_MAX_FIXED 20
+typedef struct alore_task {
+  int32_t n_objects;          /* n >= 1; points 0 robot, 1..n objects, n+1..2n targets */
+  int32_t fixed_assignment;   /* 1: object i goes to assign[i-1]; 0: assignment searched too */
+  const int32_t* assign;      /* [n] host, fixed mode only; NULL = i -> n+i */
+  const int32_t* leg_from;    /* [B] host; -1 = not a task leg */
+  const int32_t* leg_to;      /* [B] host */
+} alore_task_t;
+typedef struct alore_task_plan {
+  double cost;                /* optimum of the left fold; +inf when infeasible */
+  int32_t feasible, reserved;
+  int32_t* order;             /* [n] object picked k-th */
+  int32_t* target;            /* [n] where it is placed */
+  int32_t* leg_cand;          /* [2n] candidate used for each leg, tour order */
+  double* leg_cost;           /* [P*P] or NULL: the matrix D */
+  int32_t* leg_best;          /* [P*P] or NULL: its candidate indices, -1 = none */
+} alore_task_plan_t;
+/* host cost/ok [B]: results of alore_opt_batch or alore_multi_opt_batch.  Uploads them, then runs exactly the kernels
+ * of the batch entry point below. */
+int alore_task_plan(alore_ctx* ctx, const alore_task_t* task, int B, const double* cost, const int32_t* ok,
+                    alore_task_plan_t* out);
+/* the device results of the last run of `batch` (nothing of the batch is downloaded); waits for the device first, as
+ * the batch argmin does.  leg_from/leg_to have the batch's B entries. */
+int alore_batch_task_plan(alore_ctx* ctx, alore_batch* batch, const alore_task_t* task, alore_task_plan_t* out);
+
 /* ---- several GPUs of one box behind one object (SURVEY.md section 8b ownership row, 8e) -------------------------------
  * The reference's caller is one C++ process (PlanManager, plan_manager.hpp:120-123, :662-670); alore_multi gives it the
  * multi-GPU path without a launcher: one host thread per device inside the library, the ESDF replicated (every device
