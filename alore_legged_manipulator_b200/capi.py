@@ -110,6 +110,8 @@ class TaskPlanOut(C.Structure):
 
 ALORE_TASK_MAX_FREE = 12
 ALORE_TASK_MAX_FIXED = 20
+ALORE_TASK_MAX_BEAM_N = 32
+ALORE_TASK_MAX_WIDTH = 65536
 
 
 def dptr(a: np.ndarray):
@@ -325,6 +327,10 @@ def load_library(path: os.PathLike | None = None) -> C.CDLL:
         lib.alore_selftest_division.argtypes = [vp, C.c_longlong, C.c_ulonglong, C.POINTER(C.c_longlong)]
         lib.alore_task_plan.argtypes = [vp, C.POINTER(Task), C.c_int, c_double_p, c_int32_p, C.POINTER(TaskPlanOut)]
         lib.alore_batch_task_plan.argtypes = [vp, vp, C.POINTER(Task), C.POINTER(TaskPlanOut)]
+        lib.alore_task_plan_beam.argtypes = [vp, C.POINTER(Task), C.c_int, C.c_int, c_double_p, c_int32_p,
+                                             C.POINTER(TaskPlanOut), C.POINTER(C.c_int32)]
+        lib.alore_batch_task_plan_beam.argtypes = [vp, vp, C.POINTER(Task), C.c_int, C.POINTER(TaskPlanOut),
+                                                   C.POINTER(C.c_int32)]
     if path is None:
         _lib = lib
     return lib
@@ -341,6 +347,7 @@ EXPORTED_SYMBOLS = [
     "alore_final_collision_batch", "alore_selftest_division", "alore_debug_force_exact_division", "alore_debug_set_norm_guard", "alore_debug_phase_cycles", "alore_launch_count",
     "alore_create_multi", "alore_destroy_multi", "alore_multi_size", "alore_multi_ctx", "alore_multi_last_error",
     "alore_multi_esdf_update", "alore_multi_opt_batch", "alore_task_plan", "alore_batch_task_plan",
+    "alore_task_plan_beam", "alore_batch_task_plan_beam",
 ]
 
 

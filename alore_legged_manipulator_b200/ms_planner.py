@@ -40,15 +40,20 @@ class DeviceBatch:
         self.ctx.check(self.ctx.lib.alore_batch_argmin(self.ctx.h, self.h, C.byref(bc), C.byref(bi)))
         return float(bc.value), int(bi.value)
 
-    def task_plan(self, n_objects, leg_from, leg_to, fixed_assignment=False, assign=None, with_matrix=False):
+    def task_plan(self, n_objects, leg_from, leg_to, fixed_assignment=False, assign=None, with_matrix=False, width=None):
         """alore_batch_task_plan: the task plan (task_planner.TaskPlan) from the device results of the last run, one
-        leg label per candidate of this batch."""
+        leg label per candidate of this batch.  width: None = the exact solver, an int = alore_batch_task_plan_beam."""
         from .task_planner import TaskCall
         call = TaskCall(n_objects, leg_from, leg_to, fixed_assignment, assign, with_matrix)
         if call.B != self.cands.B:
             raise ValueError(f"{call.B} leg labels for a batch of {self.cands.B} candidates")
-        self.ctx.check(self.ctx.lib.alore_batch_task_plan(self.ctx.h, self.h, C.byref(call.task), C.byref(call.out)))
-        return call.result()
+        if width is None:
+            self.ctx.check(self.ctx.lib.alore_batch_task_plan(self.ctx.h, self.h, C.byref(call.task), C.byref(call.out)))
+            return call.result()
+        exact = C.c_int32(-1)
+        self.ctx.check(self.ctx.lib.alore_batch_task_plan_beam(self.ctx.h, self.h, C.byref(call.task), int(width),
+                                                               C.byref(call.out), C.byref(exact)))
+        return call.result(exact)
 
     def device_results(self):
         dc, dk = C.c_void_p(), C.c_void_p()

@@ -348,6 +348,34 @@ int alore_task_plan(alore_ctx* ctx, const alore_task_t* task, int B, const doubl
  * the batch argmin does.  leg_from/leg_to have the batch's B entries. */
 int alore_batch_task_plan(alore_ctx* ctx, alore_batch* batch, const alore_task_t* task, alore_task_plan_t* out);
 
+/* ---- task plan beyond the exact limits: bounded-width layered search with a proven-optimal flag ----------------------
+ * Everything above stays: task points, leg labels, the leg matrix D / best, the tour and its left-fold cost, the free
+ * and fixed modes, assign, and alore_task_plan_t.  Limits: 1 <= n_objects <= ALORE_TASK_MAX_BEAM_N in both modes (sets
+ * are uint32 masks: bit i of O is object point i+1, bit i of T is target point n+1+i), 1 <= width <=
+ * ALORE_TASK_MAX_WIDTH; anything else returns ALORE_EINVAL ("task plan: ...") before any launch.
+ * States are the exact DP's half-step states: A (O, T, j), j just picked, |O| = |T|+1; B (O, T, u), u just filled,
+ * |O| = |T| (fixed mode: T is the image of O).  Layer A_1 holds ({j}, {}, j) with value D[0][1+j].  A successor of a
+ * state has value fl(value + D[last][next]): an A-state's successors are the B-states it can fill (fixed mode: only
+ * u = assign(j)), a B-state's successors the A-states it can pick next.  A successor whose value is not < +inf (+inf,
+ * NaN) is dropped.  Successors of the same state (O, T, last) merge: the minimum under IEEE < (-0 and +0 tie), among
+ * equal minima the one whose predecessor's last point has the lowest index; the merged state keeps that record's exact
+ * value bits and that predecessor as its parent (the exact DP's tie rule).  If a layer has more than `width` merged
+ * states, the first `width` are kept in the total order (value with -0 == +0, then O as an unsigned integer, then T,
+ * then the local index of the last point), so the kept set is unique.  The final minimum over the last layer and the
+ * backtrack of the parents follow the exact DP (free: ascending u, fixed: ascending j); infeasible when that minimum
+ * is +inf or a layer is empty.
+ * exact (may be NULL) = 1 iff no layer had more merged states than `width`; then the result equals alore_task_plan bit
+ * for bit (cost, plan, leg_cand, matrix).  width = 1 is the greedy walk that steps to the next point minimising
+ * fl(value + D[last][next]), ties (IEEE ==) to the lowest point index.
+ * Blocking, one stream synchronise per call, no host round trip per layer; scratch in the same context arena as the
+ * exact entries, so both may alternate on one context in any size order. */
+#define ALORE_TASK_MAX_BEAM_N 32
+#define ALORE_TASK_MAX_WIDTH 65536
+int alore_task_plan_beam(alore_ctx* ctx, const alore_task_t* task, int width, int B, const double* cost, const int32_t* ok,
+                         alore_task_plan_t* out, int32_t* exact);
+int alore_batch_task_plan_beam(alore_ctx* ctx, alore_batch* batch, const alore_task_t* task, int width,
+                               alore_task_plan_t* out, int32_t* exact);
+
 /* ---- several GPUs of one box behind one object (SURVEY.md section 8b ownership row, 8e) -------------------------------
  * The reference's caller is one C++ process (PlanManager, plan_manager.hpp:120-123, :662-670); alore_multi gives it the
  * multi-GPU path without a launcher: one host thread per device inside the library, the ESDF replicated (every device
