@@ -19,6 +19,7 @@
 #include <algorithm>
 #include <climits>
 #include <cmath>
+#include <optional>
 
 #include "common.cuh"
 
@@ -512,16 +513,16 @@ unsigned long long binom_host(int n, int k) {
   return v;
 }
 
-// width = 0: the exact solver's limits; width != 0: the bounded-width search's
-int validate(alore_ctx* ctx, const alore_task_t* task, int B, const alore_task_plan_t* out, int width = 0) {
+// width: none = the exact solver's limits; a width = the bounded-width search's, the width itself checked first
+int validate(alore_ctx* ctx, const alore_task_t* task, int B, const alore_task_plan_t* out, std::optional<int> width) {
+  if (width && (*width < 1 || *width > ALORE_TASK_MAX_WIDTH))
+    return alore_fail(ctx, ALORE_EINVAL, "task plan: width %d outside [1, %d]", *width, ALORE_TASK_MAX_WIDTH);
   if (!task || !out) return alore_fail(ctx, ALORE_EINVAL, "task plan: null task or plan");
   const int fixed = task->fixed_assignment, n = task->n_objects;
   if (fixed != 0 && fixed != 1) return alore_fail(ctx, ALORE_EINVAL, "task plan: fixed_assignment must be 0 or 1, not %d", fixed);
   const int nmax = width ? ALORE_TASK_MAX_BEAM_N : fixed ? ALORE_TASK_MAX_FIXED : ALORE_TASK_MAX_FREE;
   if (n < 1 || n > nmax)
     return alore_fail(ctx, ALORE_EINVAL, "task plan: n_objects %d outside [1, %d] in %s mode", n, nmax, fixed ? "fixed" : "free");
-  if (width && (width < 1 || width > ALORE_TASK_MAX_WIDTH))
-    return alore_fail(ctx, ALORE_EINVAL, "task plan: width %d outside [1, %d]", width, ALORE_TASK_MAX_WIDTH);
   if (!out->order || !out->target || !out->leg_cand) return alore_fail(ctx, ALORE_EINVAL, "task plan: null order/target/leg_cand");
   if (B < 0) return alore_fail(ctx, ALORE_EINVAL, "task plan: negative batch size");
   if (B > 0 && (!task->leg_from || !task->leg_to)) return alore_fail(ctx, ALORE_EINVAL, "task plan: null leg labels");
@@ -546,257 +547,271 @@ int validate(alore_ctx* ctx, const alore_task_t* task, int B, const alore_task_p
   return ALORE_OK;
 }
 
-// Carves aligned pieces from the context's task arena.
+// Carves aligned pieces from the context's task arena at `base`.  From base 0 it only measures: `at` is then the bytes
+// the layout needs, so one layout both sizes the arena and points into it.  A carve only stores the pieces it takes;
+// pointers derived from them are formed once the arena is in place.
 struct Carve {
+  uintptr_t base = 0;
   size_t at = 0;
   template <class T>
-  size_t take(size_t n) {
+  T* take(size_t n) {
     const size_t o = (at + 255) & ~size_t(255);
     at = o + n * sizeof(T);
-    return o;
+    return reinterpret_cast<T*>(base + o);
   }
 };
 
-// The one device path.  d_cost/d_ok: device results (batch entry), or NULL with h_cost/h_ok to upload (host entry).
-// width = 0: the exact DP; width >= 1: the bounded-width search, its `exact` flag to *exact (may be NULL).
-int task_plan_run(alore_ctx* ctx, const alore_task_t* task, int B, const double* d_cost, const int32_t* d_ok,
-                  const double* h_cost, const int32_t* h_ok, alore_task_plan_t* out, int width = 0, int32_t* exact = nullptr) {
-  const int n = task->n_objects, P = 2 * n + 1, PP = P * P;
-  const bool fixed = task->fixed_assignment == 1;
-  int8_t tgt[kBeamN];
-  for (int i = 0; i < n; i++) tgt[i] = (int8_t)((fixed && task->assign ? task->assign[i] : n + 1 + i) - n - 1);
-  TaskDP dp{};
-  long long S = 0;
-  if (!width) {
-    dp.n = n;
-    dp.P = P;
+// local target (0..n-1) of local object i
+int8_t local_target(const alore_task_t& task, int i) {
+  const int n = task.n_objects;
+  return (int8_t)((task.fixed_assignment == 1 && task.assign ? task.assign[i] : n + 1 + i) - n - 1);
+}
+
+// What both solvers share: the output block, downloaded in one copy,
+//   [D PP][cost][feasible, order n, target n, leg_cand 2n, (exact)][best PP]
+// and the leg-matrix scratch, at the front of the arena.  cost/ok: the device results of a batch, or NULL and
+// h_cost/h_ok are uploaded into the arena.  flags: ints after the plan (the bounded-width search's `exact`).
+struct TaskFront {
+  const alore_task_t& task;
+  int n, P, PP, B;
+  size_t n_ints, block_bytes;
+  const double* h_cost;
+  const int32_t* h_ok;
+  const double* cost;
+  const int32_t* ok;
+  char* block = nullptr;
+  unsigned long long* key = nullptr;
+  int32_t *from = nullptr, *to = nullptr;
+  TaskFront(const alore_task_t& task, int B, const double* d_cost, const int32_t* d_ok, const double* h_cost,
+            const int32_t* h_ok, int flags)
+      : task(task), n(task.n_objects), P(2 * n + 1), PP(P * P), B(B), n_ints(1 + 4 * (size_t)n + flags),
+        block_bytes(8 * (size_t)PP + 8 + 4 * (n_ints + PP)), h_cost(h_cost), h_ok(h_ok), cost(d_cost), ok(d_ok) {}
+  void carve(Carve& cv) {
+    block = cv.take<char>(block_bytes);
+    key = cv.take<unsigned long long>(PP);
+    from = cv.take<int32_t>(B);
+    to = cv.take<int32_t>(B);
+    if (h_cost) {
+      cost = cv.take<double>(B);
+      ok = cv.take<int32_t>(B);
+    }
+  }
+  double* D() const { return reinterpret_cast<double*>(block); }
+  double* opt() const { return D() + PP; }
+  int32_t* ints() const { return reinterpret_cast<int32_t*>(opt() + 1); }
+  int32_t* best() const { return ints() + n_ints; }
+  // uploads the labels (and host cost / ok) and builds the leg matrix D and its candidate indices
+  int leg_matrix(alore_ctx* ctx) const {
+    cudaStream_t st = ctx->stream;
+    ALORE_CUDA(ctx, cudaMemsetAsync(key, 0xFF, PP * sizeof(unsigned long long), st));   // key = max
+    ALORE_CUDA(ctx, cudaMemsetAsync(best(), 0x7F, PP * sizeof(int32_t), st));           // index = 0x7F7F7F7F
+    if (B > 0) {
+      ALORE_CUDA(ctx, cudaMemcpyAsync(from, task.leg_from, B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+      ALORE_CUDA(ctx, cudaMemcpyAsync(to, task.leg_to, B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+      if (h_cost) {
+        ALORE_CUDA(ctx, cudaMemcpyAsync(const_cast<double*>(cost), h_cost, B * sizeof(double), cudaMemcpyHostToDevice, st));
+        ALORE_CUDA(ctx, cudaMemcpyAsync(const_cast<int32_t*>(ok), h_ok, B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+      }
+      const int g = std::min((B + kThreads - 1) / kThreads, ctx->sm_count * 8);
+      task_leg_key_kernel<<<g, kThreads, 0, st>>>(B, P, from, to, cost, ok, key);
+      task_leg_index_kernel<<<g, kThreads, 0, st>>>(B, P, from, to, cost, ok, key, best());
+      ctx->launches += 2;
+    }
+    task_leg_final_kernel<<<(PP + kThreads - 1) / kThreads, kThreads, 0, st>>>(B, P, cost, best(), D());
+    ctx->launches++;
+    return ALORE_OK;
+  }
+  // downloads the plan, and the matrix only when it is asked for; the call's one synchronise.  exact: the flag after
+  // the plan, NULL when there is none.
+  int read_back(alore_ctx* ctx, alore_task_plan_t* out, int32_t* exact) const {
+    const bool with_matrix = out->leg_cost || out->leg_best;
+    std::vector<char> h(block_bytes);
+    const size_t lo = with_matrix ? 0 : 8 * (size_t)PP, hi = with_matrix ? block_bytes : 8 * (size_t)PP + 8 + 4 * n_ints;
+    ALORE_CUDA(ctx, cudaMemcpyAsync(h.data() + lo, block + lo, hi - lo, cudaMemcpyDeviceToHost, ctx->stream));
+    ALORE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    const double* hD = reinterpret_cast<const double*>(h.data());
+    const int32_t* hi32 = reinterpret_cast<const int32_t*>(hD + PP + 1);
+    std::memcpy(&out->cost, hD + PP, sizeof(double));
+    out->feasible = hi32[0];
+    std::memcpy(out->order, hi32 + 1, n * sizeof(int32_t));
+    std::memcpy(out->target, hi32 + 1 + n, n * sizeof(int32_t));
+    std::memcpy(out->leg_cand, hi32 + 1 + 2 * n, 2 * n * sizeof(int32_t));
+    if (out->leg_cost) std::memcpy(out->leg_cost, hD, PP * sizeof(double));
+    if (out->leg_best) std::memcpy(out->leg_best, hi32 + n_ints, PP * sizeof(int32_t));
+    if (exact) *exact = hi32[1 + 4 * n];
+    return ALORE_OK;
+  }
+};
+
+// The exact layered DP: a value and a parent per state of every layer.
+struct ExactSolve {
+  static constexpr int kFlags = 0;
+  TaskDP p{};
+  long long S = 0;                                           // states of all layers
+  bool fixed;
+  explicit ExactSolve(const alore_task_t& task) : fixed(task.fixed_assignment == 1) {
+    const int n = task.n_objects;
+    p.n = n;
+    p.P = 2 * n + 1;
     for (int k = 1; k <= n; k++) {
       const unsigned long long cO = binom_host(n, k);
-      dp.off[2 * k - 2] = S;
+      p.off[2 * k - 2] = S;
       S += (long long)(cO * (fixed ? 1 : binom_host(n, k - 1)) * k);
-      dp.off[2 * k - 1] = S;
+      p.off[2 * k - 1] = S;
       S += (long long)(cO * (fixed ? 1 : cO) * k);
     }
     for (int i = 0; i < n; i++) {
-      dp.tgt[i] = tgt[i];
-      dp.obj[tgt[i]] = (int8_t)i;
+      p.tgt[i] = local_target(task, i);
+      p.obj[p.tgt[i]] = (int8_t)i;
     }
   }
-  // bounded-width search: at most W n successors per layer, hash tables at load <= 1/2
-  TaskBeam bm{};
-  bm.n = n;
-  bm.P = P;
-  bm.W = width;
-  const size_t E = (size_t)width * n;
-  bm.H = 256;
-  while (width && (size_t)bm.H < 2 * E) bm.H *= 2;
-  std::memcpy(bm.tgt, tgt, sizeof(tgt));
-  // output block (one contiguous download): [D PP][cost][feasible, order n, target n, leg_cand 2n, (exact)][best PP]
-  const size_t n_ints = 1 + 4 * (size_t)n + (width ? 1 : 0);
-  const size_t block_bytes = 8 * (size_t)PP + 8 + 4 * (n_ints + PP);
-  Carve cv;
-  const size_t o_block = cv.take<char>(block_bytes);
-  const size_t o_key = cv.take<unsigned long long>(PP);
-  const size_t o_from = cv.take<int32_t>(B), o_to = cv.take<int32_t>(B);
-  const size_t o_cost = h_cost ? cv.take<double>(B) : 0, o_ok = h_cost ? cv.take<int32_t>(B) : 0;
-  const size_t o_val = cv.take<double>(S), o_par = cv.take<int8_t>(S);
-  size_t o_tab = 0, o_m[6] = {}, o_k[2][4] = {}, o_blast = 0, o_bpar = 0, o_ctl = 0;
-  if (width) {
-    const size_t W = width;
-    o_tab = cv.take<unsigned long long>(4 * (size_t)bm.H);   // key1, key2 (cleared to 0), vkey, pred (set to ~0)
-    o_m[0] = cv.take<unsigned long long>(E);
-    o_m[1] = cv.take<uint32_t>(E);
-    o_m[2] = cv.take<uint32_t>(E);
-    o_m[3] = cv.take<int32_t>(E);
-    o_m[4] = cv.take<int8_t>(E);
-    o_m[5] = cv.take<double>(E);
-    for (int b = 0; b < 2; b++) {
-      o_k[b][0] = cv.take<uint32_t>(W);
-      o_k[b][1] = cv.take<uint32_t>(W);
-      o_k[b][2] = cv.take<int8_t>(W);
-      o_k[b][3] = cv.take<double>(W);
-    }
-    o_blast = cv.take<int8_t>(2 * n * W);
-    o_bpar = cv.take<int32_t>(2 * n * W);
-    o_ctl = cv.take<BeamCtl>(1);
+  void carve(Carve& cv) {
+    p.val = cv.take<double>(S);
+    p.par = cv.take<int8_t>(S);
   }
-  const size_t need = cv.at;
+  int enqueue(alore_ctx* ctx, const TaskFront& f) {
+    cudaStream_t st = ctx->stream;
+    p.D = f.D();
+    for (int k = 1; k <= p.n; k++) {
+      const long long nA = p.off[2 * k - 1] - p.off[2 * k - 2];
+      const long long nB = (k < p.n ? p.off[2 * k] : S) - p.off[2 * k - 1];
+      const int gA = (int)std::min<long long>((nA + kThreads - 1) / kThreads, ctx->sm_count * 8LL);
+      const int gB = (int)std::min<long long>((nB + kThreads - 1) / kThreads, ctx->sm_count * 8LL);
+      if (fixed) {
+        task_pick_kernel<true><<<gA, kThreads, 0, st>>>(p, k);
+        task_place_kernel<true><<<gB, kThreads, 0, st>>>(p, k);
+      } else {
+        task_pick_kernel<false><<<gA, kThreads, 0, st>>>(p, k);
+        task_place_kernel<false><<<gB, kThreads, 0, st>>>(p, k);
+      }
+      ctx->launches += 2;
+    }
+    if (fixed) task_backtrack_kernel<true><<<1, 32, 0, st>>>(p, f.best(), f.opt(), f.ints());
+    else task_backtrack_kernel<false><<<1, 32, 0, st>>>(p, f.best(), f.opt(), f.ints());
+    ctx->launches++;
+    return ALORE_OK;
+  }
+};
 
-  ALORE_CUDA(ctx, cudaSetDevice(ctx->device));
-  cudaStream_t st = ctx->stream;
-  if (need > ctx->task_pool_bytes) {
-    ALORE_CUDA(ctx, cudaStreamSynchronize(st));
-    if (ctx->task_pool) cudaFree(ctx->task_pool);
-    ctx->task_pool = nullptr;
-    ctx->task_pool_bytes = 0;
-    if (cudaMalloc(&ctx->task_pool, need) != cudaSuccess) {
-      (void)cudaGetLastError();
-      return alore_fail(ctx, ALORE_ENOMEM, "task plan: cudaMalloc of %zu bytes of scratch failed", need);
-    }
-    ctx->task_pool_bytes = need;
+// The bounded-width search: at most W n successors per layer, hash tables at load <= 1/2, and every layer's kept last
+// points and parents for the backtrack.
+struct BeamSolve {
+  static constexpr int kFlags = 1;                           // the `exact` flag after the plan
+  TaskBeam p{};
+  size_t E;
+  bool fixed;
+  unsigned long long* tab = nullptr;                         // key1, key2 (cleared to 0), vkey, pred (set to ~0)
+  BeamSolve(const alore_task_t& task, int width) : E((size_t)width * task.n_objects), fixed(task.fixed_assignment == 1) {
+    p.n = task.n_objects;
+    p.P = 2 * p.n + 1;
+    p.W = width;
+    p.H = 256;
+    while ((size_t)p.H < 2 * E) p.H *= 2;
+    for (int i = 0; i < p.n; i++) p.tgt[i] = local_target(task, i);
   }
-  char* base = static_cast<char*>(ctx->task_pool);
-  double* d_D = reinterpret_cast<double*>(base + o_block);
-  double* d_opt = d_D + PP;
-  int32_t* d_ints = reinterpret_cast<int32_t*>(d_opt + 1);
-  int32_t* d_best = d_ints + n_ints;
-  auto* d_key = reinterpret_cast<unsigned long long*>(base + o_key);
-  auto* d_from = reinterpret_cast<int32_t*>(base + o_from);
-  auto* d_to = reinterpret_cast<int32_t*>(base + o_to);
-  if (h_cost) {
-    d_cost = reinterpret_cast<double*>(base + o_cost);
-    d_ok = reinterpret_cast<int32_t*>(base + o_ok);
-  }
-  dp.D = d_D;
-  dp.val = reinterpret_cast<double*>(base + o_val);
-  dp.par = reinterpret_cast<int8_t*>(base + o_par);
-  if (width) {
-    bm.D = d_D;
-    auto* tab = reinterpret_cast<unsigned long long*>(base + o_tab);
-    bm.key1 = tab;
-    bm.key2 = tab + bm.H;
-    bm.vkey = tab + 2 * (size_t)bm.H;
-    bm.pred = tab + 3 * (size_t)bm.H;
-    bm.mkey = reinterpret_cast<unsigned long long*>(base + o_m[0]);
-    bm.mO = reinterpret_cast<uint32_t*>(base + o_m[1]);
-    bm.mT = reinterpret_cast<uint32_t*>(base + o_m[2]);
-    bm.mpar = reinterpret_cast<int32_t*>(base + o_m[3]);
-    bm.mlast = reinterpret_cast<int8_t*>(base + o_m[4]);
-    bm.mval = reinterpret_cast<double*>(base + o_m[5]);
+  void carve(Carve& cv) {
+    const size_t W = p.W;
+    tab = cv.take<unsigned long long>(4 * (size_t)p.H);
+    p.mkey = cv.take<unsigned long long>(E);
+    p.mO = cv.take<uint32_t>(E);
+    p.mT = cv.take<uint32_t>(E);
+    p.mpar = cv.take<int32_t>(E);
+    p.mlast = cv.take<int8_t>(E);
+    p.mval = cv.take<double>(E);
     for (int b = 0; b < 2; b++) {
-      bm.kO[b] = reinterpret_cast<uint32_t*>(base + o_k[b][0]);
-      bm.kT[b] = reinterpret_cast<uint32_t*>(base + o_k[b][1]);
-      bm.klast[b] = reinterpret_cast<int8_t*>(base + o_k[b][2]);
-      bm.kval[b] = reinterpret_cast<double*>(base + o_k[b][3]);
+      p.kO[b] = cv.take<uint32_t>(W);
+      p.kT[b] = cv.take<uint32_t>(W);
+      p.klast[b] = cv.take<int8_t>(W);
+      p.kval[b] = cv.take<double>(W);
     }
-    bm.blast = reinterpret_cast<int8_t*>(base + o_blast);
-    bm.bpar = reinterpret_cast<int32_t*>(base + o_bpar);
-    bm.ctl = reinterpret_cast<BeamCtl*>(base + o_ctl);
-    ALORE_CUDA(ctx, cudaMemsetAsync(bm.key1, 0, 2 * (size_t)bm.H * sizeof(unsigned long long), st));
-    ALORE_CUDA(ctx, cudaMemsetAsync(bm.vkey, 0xFF, 2 * (size_t)bm.H * sizeof(unsigned long long), st));
-    ALORE_CUDA(ctx, cudaMemsetAsync(bm.ctl, 0, sizeof(BeamCtl), st));
+    p.blast = cv.take<int8_t>(2 * p.n * W);
+    p.bpar = cv.take<int32_t>(2 * p.n * W);
+    p.ctl = cv.take<BeamCtl>(1);
   }
-
-  ALORE_CUDA(ctx, cudaMemsetAsync(d_key, 0xFF, PP * sizeof(unsigned long long), st));   // key = max
-  ALORE_CUDA(ctx, cudaMemsetAsync(d_best, 0x7F, PP * sizeof(int32_t), st));            // index = 0x7F7F7F7F
-  if (B > 0) {
-    ALORE_CUDA(ctx, cudaMemcpyAsync(d_from, task->leg_from, B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    ALORE_CUDA(ctx, cudaMemcpyAsync(d_to, task->leg_to, B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    if (h_cost) {
-      ALORE_CUDA(ctx, cudaMemcpyAsync(const_cast<double*>(d_cost), h_cost, B * sizeof(double), cudaMemcpyHostToDevice, st));
-      ALORE_CUDA(ctx, cudaMemcpyAsync(const_cast<int32_t*>(d_ok), h_ok, B * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-    }
-    const int g = std::min((B + kThreads - 1) / kThreads, ctx->sm_count * 8);
-    task_leg_key_kernel<<<g, kThreads, 0, st>>>(B, P, d_from, d_to, d_cost, d_ok, d_key);
-    task_leg_index_kernel<<<g, kThreads, 0, st>>>(B, P, d_from, d_to, d_cost, d_ok, d_key, d_best);
-    ctx->launches += 2;
-  }
-  task_leg_final_kernel<<<(PP + kThreads - 1) / kThreads, kThreads, 0, st>>>(B, P, d_cost, d_best, d_D);
-  ctx->launches++;
-  if (width) {
+  int enqueue(alore_ctx* ctx, const TaskFront& f) {
+    cudaStream_t st = ctx->stream;
+    p.D = f.D();
+    p.key1 = tab;
+    p.key2 = tab + p.H;
+    p.vkey = tab + 2 * (size_t)p.H;
+    p.pred = tab + 3 * (size_t)p.H;
+    ALORE_CUDA(ctx, cudaMemsetAsync(p.key1, 0, 2 * (size_t)p.H * sizeof(unsigned long long), st));
+    ALORE_CUDA(ctx, cudaMemsetAsync(p.vkey, 0xFF, 2 * (size_t)p.H * sizeof(unsigned long long), st));
+    ALORE_CUDA(ctx, cudaMemsetAsync(p.ctl, 0, sizeof(BeamCtl), st));
     const long long cap = ctx->sm_count * 8LL;
     const int gE = (int)std::min<long long>(((long long)E + kThreads - 1) / kThreads, cap);
-    const int gH = (int)std::min<long long>(bm.H / kThreads, cap);
-    for (int l = 1; l <= 2 * n; l++) {
+    const int gH = (int)std::min<long long>(p.H / kThreads, cap);
+    for (int l = 1; l <= 2 * p.n; l++) {
       if (fixed) {
-        task_beam_expand_kernel<true, 1><<<gE, kThreads, 0, st>>>(bm, l);
-        task_beam_expand_kernel<true, 2><<<gE, kThreads, 0, st>>>(bm, l);
+        task_beam_expand_kernel<true, 1><<<gE, kThreads, 0, st>>>(p, l);
+        task_beam_expand_kernel<true, 2><<<gE, kThreads, 0, st>>>(p, l);
       } else {
-        task_beam_expand_kernel<false, 1><<<gE, kThreads, 0, st>>>(bm, l);
-        task_beam_expand_kernel<false, 2><<<gE, kThreads, 0, st>>>(bm, l);
+        task_beam_expand_kernel<false, 1><<<gE, kThreads, 0, st>>>(p, l);
+        task_beam_expand_kernel<false, 2><<<gE, kThreads, 0, st>>>(p, l);
       }
-      task_beam_merge_kernel<<<gH, kThreads, 0, st>>>(bm, l);
-      for (int d = 0; d < kBeamDigits; d++) task_beam_select_kernel<<<gE, kThreads, 0, st>>>(bm, l, d);
-      task_beam_keep_kernel<<<gH, kThreads, 0, st>>>(bm, l);
+      task_beam_merge_kernel<<<gH, kThreads, 0, st>>>(p, l);
+      for (int d = 0; d < kBeamDigits; d++) task_beam_select_kernel<<<gE, kThreads, 0, st>>>(p, l, d);
+      task_beam_keep_kernel<<<gH, kThreads, 0, st>>>(p, l);
       ctx->launches += 4 + kBeamDigits;
     }
-    if (fixed) task_beam_backtrack_kernel<true><<<1, 32, 0, st>>>(bm, d_best, d_opt, d_ints);
-    else task_beam_backtrack_kernel<false><<<1, 32, 0, st>>>(bm, d_best, d_opt, d_ints);
+    if (fixed) task_beam_backtrack_kernel<true><<<1, 32, 0, st>>>(p, f.best(), f.opt(), f.ints());
+    else task_beam_backtrack_kernel<false><<<1, 32, 0, st>>>(p, f.best(), f.opt(), f.ints());
     ctx->launches++;
+    return ALORE_OK;
   }
-  for (int k = 1; k <= n && !width; k++) {
-    const long long nA = dp.off[2 * k - 1] - dp.off[2 * k - 2];
-    const long long nB = (k < n ? dp.off[2 * k] : S) - dp.off[2 * k - 1];
-    const int gA = (int)std::min<long long>((nA + kThreads - 1) / kThreads, ctx->sm_count * 8LL);
-    const int gB = (int)std::min<long long>((nB + kThreads - 1) / kThreads, ctx->sm_count * 8LL);
-    if (fixed) {
-      task_pick_kernel<true><<<gA, kThreads, 0, st>>>(dp, k);
-      task_place_kernel<true><<<gB, kThreads, 0, st>>>(dp, k);
-    } else {
-      task_pick_kernel<false><<<gA, kThreads, 0, st>>>(dp, k);
-      task_place_kernel<false><<<gB, kThreads, 0, st>>>(dp, k);
+};
+
+// The one device path: the shared front end and the solver's own scratch carved from the context's arena (grown only
+// when a call needs more), the leg matrix, the solver's layers, and the shared read-back.  d_cost/d_ok: device results (batch entries), or NULL with h_cost/h_ok to
+// upload (host entries).  width: none = the exact DP; a width = the bounded-width search, its `exact` flag to *exact
+// (may be NULL).
+int task_plan_run(alore_ctx* ctx, const alore_task_t* task, int B, const double* d_cost, const int32_t* d_ok,
+                  const double* h_cost, const int32_t* h_ok, alore_task_plan_t* out, std::optional<int> width,
+                  int32_t* exact) {
+  auto run = [&](auto solve, int32_t* flag) {
+    TaskFront f(*task, B, d_cost, d_ok, h_cost, h_ok, decltype(solve)::kFlags);
+    Carve size;
+    f.carve(size);
+    solve.carve(size);
+    ALORE_CUDA(ctx, cudaSetDevice(ctx->device));
+    if (size.at > ctx->task_pool_bytes) {                   // the synchronise keeps the old arena until its work is done
+      ALORE_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+      if (ctx->task_pool) cudaFree(ctx->task_pool);
+      ctx->task_pool = nullptr;
+      ctx->task_pool_bytes = 0;
+      if (cudaMalloc(&ctx->task_pool, size.at) != cudaSuccess) {
+        (void)cudaGetLastError();
+        return alore_fail(ctx, ALORE_ENOMEM, "task plan: cudaMalloc of %zu bytes of scratch failed", size.at);
+      }
+      ctx->task_pool_bytes = size.at;
     }
-    ctx->launches += 2;
-  }
-  if (!width) {
-    if (fixed) task_backtrack_kernel<true><<<1, 32, 0, st>>>(dp, d_best, d_opt, d_ints);
-    else task_backtrack_kernel<false><<<1, 32, 0, st>>>(dp, d_best, d_opt, d_ints);
-    ctx->launches++;
-  }
-  ALORE_CUDA(ctx, cudaGetLastError());
-
-  // download the plan, and the matrix only when it is asked for
-  const bool with_matrix = out->leg_cost || out->leg_best;
-  std::vector<char> h(block_bytes);
-  const size_t lo = with_matrix ? 0 : 8 * (size_t)PP, hi = with_matrix ? block_bytes : 8 * (size_t)PP + 8 + 4 * n_ints;
-  ALORE_CUDA(ctx, cudaMemcpyAsync(h.data() + lo, base + o_block + lo, hi - lo, cudaMemcpyDeviceToHost, st));
-  ALORE_CUDA(ctx, cudaStreamSynchronize(st));
-  const double* hD = reinterpret_cast<const double*>(h.data());
-  const int32_t* hi32 = reinterpret_cast<const int32_t*>(hD + PP + 1);
-  std::memcpy(&out->cost, hD + PP, sizeof(double));
-  out->feasible = hi32[0];
-  std::memcpy(out->order, hi32 + 1, n * sizeof(int32_t));
-  std::memcpy(out->target, hi32 + 1 + n, n * sizeof(int32_t));
-  std::memcpy(out->leg_cand, hi32 + 1 + 2 * n, 2 * n * sizeof(int32_t));
-  if (out->leg_cost) std::memcpy(out->leg_cost, hD, PP * sizeof(double));
-  if (out->leg_best) std::memcpy(out->leg_best, hi32 + n_ints, PP * sizeof(int32_t));
-  if (width && exact) *exact = hi32[1 + 4 * n];
-  return ALORE_OK;
+    Carve cv{reinterpret_cast<uintptr_t>(ctx->task_pool)};
+    f.carve(cv);
+    solve.carve(cv);
+    int rc = f.leg_matrix(ctx);
+    if (rc) return rc;
+    if ((rc = solve.enqueue(ctx, f))) return rc;
+    ALORE_CUDA(ctx, cudaGetLastError());
+    return f.read_back(ctx, out, flag);
+  };
+  if (width) return run(BeamSolve(*task, *width), exact);
+  return run(ExactSolve(*task), nullptr);
 }
 
-}  // namespace
-
-extern "C" {
-
-int alore_task_plan(alore_ctx* ctx, const alore_task_t* task, int B, const double* cost, const int32_t* ok,
-                    alore_task_plan_t* out) {
+// alore_task_plan and alore_task_plan_beam: cost / ok in host memory
+int host_plan(alore_ctx* ctx, const alore_task_t* task, std::optional<int> width, int B, const double* cost,
+              const int32_t* ok, alore_task_plan_t* out, int32_t* exact) {
   if (!ctx) return ALORE_EINVAL;
-  int rc = validate(ctx, task, B, out);
-  if (rc) return rc;
-  if (B > 0 && (!cost || !ok)) return alore_fail(ctx, ALORE_EINVAL, "task plan: null cost/ok");
-  return task_plan_run(ctx, task, B, nullptr, nullptr, cost, ok, out);
-}
-
-int alore_batch_task_plan(alore_ctx* ctx, alore_batch* batch, const alore_task_t* task, alore_task_plan_t* out) {
-  if (!ctx || !batch) return ALORE_EINVAL;
-  int B = 0, runs = 0;
-  const double* d_cost = nullptr;
-  const int32_t* d_ok = nullptr;
-  batch_result_view(batch, &B, &runs, &d_cost, &d_ok);
-  int rc = validate(ctx, task, B, out);
-  if (rc) return rc;
-  if (runs == 0) return alore_fail(ctx, ALORE_EINVAL, "task plan: the batch has not been run");
-  ALORE_CUDA(ctx, cudaSetDevice(ctx->device));
-  ALORE_CUDA(ctx, cudaDeviceSynchronize());                 // the run may have been enqueued on a caller stream
-  return task_plan_run(ctx, task, B, d_cost, d_ok, nullptr, nullptr, out);
-}
-
-int alore_task_plan_beam(alore_ctx* ctx, const alore_task_t* task, int width, int B, const double* cost, const int32_t* ok,
-                         alore_task_plan_t* out, int32_t* exact) {
-  if (!ctx) return ALORE_EINVAL;
-  if (width < 1 || width > ALORE_TASK_MAX_WIDTH)
-    return alore_fail(ctx, ALORE_EINVAL, "task plan: width %d outside [1, %d]", width, ALORE_TASK_MAX_WIDTH);
   int rc = validate(ctx, task, B, out, width);
   if (rc) return rc;
   if (B > 0 && (!cost || !ok)) return alore_fail(ctx, ALORE_EINVAL, "task plan: null cost/ok");
   return task_plan_run(ctx, task, B, nullptr, nullptr, cost, ok, out, width, exact);
 }
 
-int alore_batch_task_plan_beam(alore_ctx* ctx, alore_batch* batch, const alore_task_t* task, int width,
-                               alore_task_plan_t* out, int32_t* exact) {
+// alore_batch_task_plan and alore_batch_task_plan_beam: the device results of the batch's last run
+int batch_plan(alore_ctx* ctx, alore_batch* batch, const alore_task_t* task, std::optional<int> width,
+               alore_task_plan_t* out, int32_t* exact) {
   if (!ctx || !batch) return ALORE_EINVAL;
-  if (width < 1 || width > ALORE_TASK_MAX_WIDTH)
-    return alore_fail(ctx, ALORE_EINVAL, "task plan: width %d outside [1, %d]", width, ALORE_TASK_MAX_WIDTH);
   int B = 0, runs = 0;
   const double* d_cost = nullptr;
   const int32_t* d_ok = nullptr;
@@ -807,6 +822,29 @@ int alore_batch_task_plan_beam(alore_ctx* ctx, alore_batch* batch, const alore_t
   ALORE_CUDA(ctx, cudaSetDevice(ctx->device));
   ALORE_CUDA(ctx, cudaDeviceSynchronize());                 // the run may have been enqueued on a caller stream
   return task_plan_run(ctx, task, B, d_cost, d_ok, nullptr, nullptr, out, width, exact);
+}
+
+}  // namespace
+
+extern "C" {
+
+int alore_task_plan(alore_ctx* ctx, const alore_task_t* task, int B, const double* cost, const int32_t* ok,
+                    alore_task_plan_t* out) {
+  return host_plan(ctx, task, std::nullopt, B, cost, ok, out, nullptr);
+}
+
+int alore_batch_task_plan(alore_ctx* ctx, alore_batch* batch, const alore_task_t* task, alore_task_plan_t* out) {
+  return batch_plan(ctx, batch, task, std::nullopt, out, nullptr);
+}
+
+int alore_task_plan_beam(alore_ctx* ctx, const alore_task_t* task, int width, int B, const double* cost, const int32_t* ok,
+                         alore_task_plan_t* out, int32_t* exact) {
+  return host_plan(ctx, task, width, B, cost, ok, out, exact);
+}
+
+int alore_batch_task_plan_beam(alore_ctx* ctx, alore_batch* batch, const alore_task_t* task, int width,
+                               alore_task_plan_t* out, int32_t* exact) {
+  return batch_plan(ctx, batch, task, width, out, exact);
 }
 
 }  // extern "C"

@@ -47,13 +47,9 @@ class DeviceBatch:
         call = TaskCall(n_objects, leg_from, leg_to, fixed_assignment, assign, with_matrix)
         if call.B != self.cands.B:
             raise ValueError(f"{call.B} leg labels for a batch of {self.cands.B} candidates")
-        if width is None:
-            self.ctx.check(self.ctx.lib.alore_batch_task_plan(self.ctx.h, self.h, C.byref(call.task), C.byref(call.out)))
-            return call.result()
-        exact = C.c_int32(-1)
-        self.ctx.check(self.ctx.lib.alore_batch_task_plan_beam(self.ctx.h, self.h, C.byref(call.task), int(width),
-                                                               C.byref(call.out), C.byref(exact)))
-        return call.result(exact)
+        ctx, lib = self.ctx, self.ctx.lib
+        return call.run(ctx, width, lambda task, out: lib.alore_batch_task_plan(ctx.h, self.h, task, out),
+                        lambda task, w, out, exact: lib.alore_batch_task_plan_beam(ctx.h, self.h, task, w, out, exact))
 
     def device_results(self):
         dc, dk = C.c_void_p(), C.c_void_p()

@@ -74,6 +74,16 @@ class TaskCall:
                         None if self.leg_best is None else self.leg_best.copy(),
                         None if exact is None else bool(exact.value))
 
+    def run(self, ctx: capi.Context, width, plan, plan_beam) -> TaskPlan:
+        """One call of the exact solver (width None) or of the bounded-width search with that width.  plan(task, out)
+        and plan_beam(task, width, out, exact) are the library's entry points with their other arguments bound."""
+        if width is None:
+            ctx.check(plan(C.byref(self.task), C.byref(self.out)))
+            return self.result()
+        exact = C.c_int32(-1)
+        ctx.check(plan_beam(C.byref(self.task), int(width), C.byref(self.out), C.byref(exact)))
+        return self.result(exact)
+
 
 def plan_tasks(ctx: capi.Context, n_objects, leg_from, leg_to, cost, ok, fixed_assignment=False, assign=None,
                with_matrix=False, width=None) -> TaskPlan:
@@ -86,10 +96,6 @@ def plan_tasks(ctx: capi.Context, n_objects, leg_from, leg_to, cost, ok, fixed_a
     ok = np.ascontiguousarray(ok, dtype=np.int32).reshape(-1)
     if cost.size != call.B or ok.size != call.B:
         raise ValueError(f"{call.B} labels but {cost.size} costs / {ok.size} ok flags")
-    if width is None:
-        ctx.check(ctx.lib.alore_task_plan(ctx.h, C.byref(call.task), call.B, capi.dptr(cost), capi.iptr(ok), C.byref(call.out)))
-        return call.result()
-    exact = C.c_int32(-1)
-    ctx.check(ctx.lib.alore_task_plan_beam(ctx.h, C.byref(call.task), int(width), call.B, capi.dptr(cost), capi.iptr(ok),
-                                           C.byref(call.out), C.byref(exact)))
-    return call.result(exact)
+    lib, src = ctx.lib, (call.B, capi.dptr(cost), capi.iptr(ok))
+    return call.run(ctx, width, lambda task, out: lib.alore_task_plan(ctx.h, task, *src, out),
+                    lambda task, w, out, exact: lib.alore_task_plan_beam(ctx.h, task, w, *src, out, exact))

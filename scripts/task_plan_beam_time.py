@@ -33,8 +33,7 @@ import numpy as np  # noqa: E402
 import bench  # noqa: E402
 import alore_legged_manipulator_b200 as alore  # noqa: E402
 from alore_legged_manipulator_b200.ms_planner import DeviceBatch  # noqa: E402
-from task_plan_beam_util import assert_same_beam_plan, oracle_plan_beam  # noqa: E402
-from task_plan_util import task_leg_batch  # noqa: E402
+from task_plan_util import assert_same_beam_plan, oracle_plan_beam, task_leg_batch  # noqa: E402
 
 N = 32
 WIDTHS = [1, 256, 4096, 65536]

@@ -1,4 +1,4 @@
-"""Helpers of the task-plan tests: the oracle call, brute force over every tour, random matrices and labelled batches."""
+"""Helpers of the task-plan tests: both oracles, brute force over every tour, random matrices and labelled batches."""
 from __future__ import annotations
 
 import ctypes as C
@@ -22,8 +22,9 @@ _oracle = None
 
 
 def load_oracle() -> C.CDLL:
-    """The sequential task-plan oracle (tests/cpp/task_plan_oracle.cpp), compiled once into the temporary directory
-    (the tree is left untouched) with the flags of the other CPU oracle: no FMA contraction, no fast-math."""
+    """The sequential task-plan oracles orc_task_plan and orc_task_plan_beam (tests/cpp/task_plan_oracle.cpp), compiled
+    once into the temporary directory (the tree is left untouched) with the flags of the other CPU oracle: no FMA
+    contraction, no fast-math."""
     global _oracle
     if _oracle is None:
         src = ORACLE_SRC.read_bytes() + (ROOT / "include" / "alore_b200.h").read_bytes()
@@ -37,6 +38,8 @@ def load_oracle() -> C.CDLL:
         _oracle = C.CDLL(str(lib))
         _oracle.orc_task_plan.argtypes = [C.POINTER(capi.Task), C.c_int, capi.c_double_p, capi.c_int32_p,
                                           C.POINTER(capi.TaskPlanOut)]
+        _oracle.orc_task_plan_beam.argtypes = [C.POINTER(capi.Task), C.c_int, C.c_int, capi.c_double_p, capi.c_int32_p,
+                                               C.POINTER(capi.TaskPlanOut), C.POINTER(C.c_int32)]
     return _oracle
 
 
@@ -51,6 +54,17 @@ def oracle_plan(n, leg_from, leg_to, cost, ok, fixed=False, assign=None, with_ma
     rc = load_oracle().orc_task_plan(C.byref(call.task), call.B, capi.dptr(cost), capi.iptr(ok), C.byref(call.out))
     assert rc == 0
     return call.result()
+
+
+def oracle_plan_beam(n, width, leg_from, leg_to, cost, ok, fixed=False, assign=None, with_matrix=True) -> TaskPlan:
+    call = TaskCall(n, leg_from, leg_to, fixed, assign, with_matrix)
+    cost = np.ascontiguousarray(cost, dtype=np.float64)
+    ok = np.ascontiguousarray(ok, dtype=np.int32)
+    exact = C.c_int32(-1)
+    rc = load_oracle().orc_task_plan_beam(C.byref(call.task), int(width), call.B, capi.dptr(cost), capi.iptr(ok),
+                                          C.byref(call.out), C.byref(exact))
+    assert rc == 0
+    return call.result(exact)
 
 
 def targets_of(n, fixed, assign):
@@ -203,6 +217,12 @@ def assert_same_plan(a: TaskPlan, b: TaskPlan):
     if a.leg_cost is not None and b.leg_cost is not None:
         assert np.array_equal(a.leg_cost.view(np.uint64), b.leg_cost.view(np.uint64))
         assert np.array_equal(a.leg_best, b.leg_best)
+
+
+def assert_same_beam_plan(a: TaskPlan, b: TaskPlan):
+    """assert_same_plan, and the same `exact` flag."""
+    assert_same_plan(a, b)
+    assert a.exact == b.exact, (a.exact, b.exact)
 
 
 def task_legs(n):

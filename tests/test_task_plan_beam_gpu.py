@@ -10,8 +10,8 @@ import pytest
 from alore_legged_manipulator_b200 import capi, plan_tasks, workloads
 from alore_legged_manipulator_b200.ms_planner import DeviceBatch
 from alore_legged_manipulator_b200.task_planner import TaskCall
-from task_plan_beam_util import assert_same_beam_plan, oracle_plan_beam
-from task_plan_util import assert_same_plan, assert_valid_plan, random_assign, random_batch, task_leg_batch
+from task_plan_util import (assert_same_beam_plan, assert_same_plan, assert_valid_plan, oracle_plan_beam, random_assign,
+                            random_batch, task_leg_batch)
 from test_esdf_gpu import make_sdf
 
 pytestmark = pytest.mark.gpu

@@ -4,9 +4,8 @@ import numpy as np
 import pytest
 
 from alore_legged_manipulator_b200 import capi
-from task_plan_beam_util import oracle_plan_beam
 from task_plan_util import (INF, assert_same_plan, assert_valid_plan, batch_of_matrix, bits, brute_force, fold,
-                            oracle_plan, random_assign, random_batch, random_matrix)
+                            oracle_plan, oracle_plan_beam, random_assign, random_batch, random_matrix)
 
 KINDS = ["ties", "inf", "neg", "zero", "all_inf", "one_tour"]
 WIDTHS = [1, 2, 3, 7, 64, capi.ALORE_TASK_MAX_WIDTH]
