@@ -556,24 +556,18 @@ static void lpt_order(const std::vector<int32_t>& po, const int32_t* evals, std:
   for (int b = 0; b < B; b++) key[b] = (long long)(po[b + 1] - po[b]) * (evals ? std::max(1, evals[b]) : 1);
   std::stable_sort(order.begin(), order.end(), [&](int a, int b) { return key[a] > key[b]; });
 }
-// Evaluation counts to predict from, for a batch with piece offsets `po`: the previous tick's counts where the previous
-// batch had the same number of candidates and (for at least 3 in 4 of them) the same piece count at the same index —
-// a replanning planner re-optimises mostly the same legs; candidates whose piece count changed get the mean count.
-// Returns false (piece counts only) when the previous batch does not look like this one.
-static bool predicted_evals(const alore_ctx* ctx, const std::vector<int32_t>& po, std::vector<int32_t>& pred) {
+// Whether the previous tick's evaluation counts (ctx->sched_evals) predict the work of a batch with piece offsets `po`:
+// the previous batch had the same number of candidates and (for at least 3 in 4 of them) the same piece count at the
+// same index — a replanning planner re-optimises mostly the same legs.  A candidate whose piece count changed is the
+// same leg re-timed, so its previous count still predicts it (with the batch mean instead, the legs of a moved way-point
+// are handed out late and become the tail of the step: 891-911 vs 830-855 ms per bench step on a B200).
+// False: piece counts only.
+static bool prediction_applies(const alore_ctx* ctx, const std::vector<int32_t>& po) {
   const int B = (int)po.size() - 1;
   if ((int)ctx->sched_evals.size() != B || (int)ctx->sched_piece_off.size() != B + 1) return false;
-  long long same = 0, sum = 0;
-  for (int b = 0; b < B; b++) {
-    same += (po[b + 1] - po[b]) == (ctx->sched_piece_off[b + 1] - ctx->sched_piece_off[b]);
-    sum += ctx->sched_evals[b];
-  }
-  if (4 * same < 3LL * B) return false;
-  const int32_t mean = (int32_t)std::max<long long>(1, sum / B);
-  pred.resize(B);
-  for (int b = 0; b < B; b++)
-    pred[b] = (po[b + 1] - po[b]) == (ctx->sched_piece_off[b + 1] - ctx->sched_piece_off[b]) ? ctx->sched_evals[b] : mean;
-  return true;
+  long long same = 0;
+  for (int b = 0; b < B; b++) same += (po[b + 1] - po[b]) == (ctx->sched_piece_off[b + 1] - ctx->sched_piece_off[b]);
+  return 4 * same >= 3LL * B;
 }
 
 static int validate_cands(alore_ctx* ctx, const alore_candidates_t* c) {
@@ -720,10 +714,9 @@ int alore_batch_run(alore_ctx* ctx, const alore_params_t* prm, alore_batch* bh, 
     ctx->last_batch = nullptr;
   }
   {
-    std::vector<int32_t> pred;
-    if (!getenv("ALORE_NO_SCHED_PREDICTION") && predicted_evals(ctx, bh->piece_off, pred)) {
+    if (!getenv("ALORE_NO_SCHED_PREDICTION") && prediction_applies(ctx, bh->piece_off)) {
       std::vector<int> order;
-      lpt_order(bh->piece_off, pred.data(), order);
+      lpt_order(bh->piece_off, ctx->sched_evals.data(), order);
       ALORE_CUDA(ctx, cudaMemcpyAsync(bh->d_order, order.data(), bh->B * sizeof(int), cudaMemcpyHostToDevice, st));
       ALORE_CUDA(ctx, cudaStreamSynchronize(st));
       bh->predicted = true;
